@@ -2,6 +2,7 @@
 """DiffusionNetBlock forward throughput (BASELINE.json metric): Mverts/s at V=200k, K=128, C=128.
 
     python bench.py --gpus 1 --steps 20 --warmup 3            # our arm (one JSON line on rank 0)
+    python bench.py --steps 20 --dump-outputs DIR             # ... and DIR/out.npy: sampled output of the last step
     python bench.py --impl reference --steps 5 --warmup 1      # the reference's CPU path (torch-CPU port)
     torchrun ... bench.py --gpus N ...                         # one rank per GPU, one mesh per rank (weak scaling)
 
@@ -26,6 +27,8 @@ N_TORUS, M_TORUS, K_EIG, C_WIDTH = 400, 500, 128, 128
 NNZ_ROW = 7
 METRIC = "DiffusionNetBlock forward Mverts/sec at V=200k,K=128,C=128; 1/2/4/8 GPU"
 WORKLOAD = "block_fwd V=200000 K=128 C=128, 1 mesh per GPU"      # identical in both arms (config.workload)
+# --dump-outputs: the whole (V, C) output is 102 MB, so a fixed sample of 2^16 of its rows (32 MB) is written
+DUMP_ROWS, DUMP_SEED = 1 << 16, 0
 
 
 def flops_per_vertex(K, C, r=NNZ_ROW):
@@ -180,7 +183,7 @@ def run_reference(args, rank):
     import diffusion_net_b200 as dn
     V = N_TORUS * M_TORUS
     (mass, L, evals, evecs, gradX, gradY), params, x = make_workload(dn, "cpu", 0)
-    steps, warm = max(1, args.steps), max(1, args.warmup)
+    steps, warm = args.steps, max(1, args.warmup)
     sec, cores, kind, sweep = time_cpu_baseline((mass, L, evals, evecs, gradX, gradY, x), params, steps, warm)
     val = V / sec / 1e6
     sample = "full workload: 1 mesh V={} K={} C={}, {} steps (median), {} warm-up; threads picked by sweep {}".format(
@@ -295,7 +298,7 @@ def run_aux(args, rank, world, local):
         dist.init_process_group("nccl", device_id=dev)
     dn.set_engine(args.engine)
     lib = dn._lib.load()
-    steps, warm = max(1, args.steps), max(3, args.warmup)
+    steps, warm = args.steps, max(3, args.warmup)
     K, C, C_in, C_out, NB = 128, 128, 16, 8, 4
 
     def barrier():
@@ -546,7 +549,15 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=8)
     ap.add_argument("--workload", default="block_fwd", choices=["block_fwd", "fwd_bwd", "train", "small_batch", "config3"],
                     help="block_fwd = the BASELINE metric (default); the others are BASELINE configs 2 / 5 / 4 / 3")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="block_fwd: after the timed steps, write the block output of the last timed step (rank 0) as "
+                         "DIR/out.npy, float32, the {} rows picked by seed {} in ascending order".format(DUMP_ROWS,
+                                                                                                         DUMP_SEED))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "block_fwd"):
+        ap.error("--dump-outputs is implemented for the block_fwd workload of our arm only")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -572,7 +583,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     lib = dn._lib.load()
     dn.set_engine(args.engine)
-    steps, warm = max(1, args.steps), max(3, args.warmup)
+    steps, warm = args.steps, max(3, args.warmup)
     V = N_TORUS * M_TORUS
 
     host_ops, params, x_host = make_workload(dn, "cpu", rank)
@@ -608,6 +619,10 @@ def main():
     barrier()
     launches = lib.dn_kernel_launch_count() - l0
     t_end = time.time()
+    dump = None
+    if args.dump_outputs and rank == 0:    # taken before the untimed steps below can touch `out`
+        rows = torch.randperm(V, generator=torch.Generator().manual_seed(DUMP_SEED))[:DUMP_ROWS].sort().values
+        dump = out[0].index_select(0, rows.to(dev))
     ms_total = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
     if world > 1:
         dist.all_reduce(ms_total, op=dist.ReduceOp.MAX)
@@ -621,6 +636,10 @@ def main():
         t_end = time.time()
     clocks = sampler.stop(t_begin, t_end)
     value = world * V / (ms_step * 1e-3) / 1e6
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "out.npy"), dump.cpu().numpy())
 
     # ---- end to end through the public API from pinned host buffers ----
     pin = lambda t: t.contiguous().pin_memory()

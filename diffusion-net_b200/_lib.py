@@ -31,12 +31,16 @@ def _stale() -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
+def nvcc() -> str:
+    """The nvcc that builds the library: $NVCC, else the CUDA toolkit's default install location."""
+    return os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+
+
 def build(force: bool = False, verbose: bool = False) -> str:
     """Compile csrc/*.cu into the in-tree shared library (nvcc cross-compiles without a GPU)."""
     if not force and not _stale():
         return LIB_PATH
-    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + ["-o", LIB_PATH] + [os.path.join(_CSRC, s) for s in SOURCES]
+    cmd = [nvcc()] + NVCC_FLAGS + ["-o", LIB_PATH] + [os.path.join(_CSRC, s) for s in SOURCES]
     if verbose:
         print(" ".join(cmd))
     r = subprocess.run(cmd, capture_output=True, text=True)

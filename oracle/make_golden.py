@@ -2,7 +2,7 @@
 
 Run in the build container only (needs /root/reference):
 
-    python oracle/make_golden.py
+    python oracle/make_golden.py [FILE ...]      # e.g. block_k128.npz: rewrite only the named fixtures
 
 Each fixture stores seeded inputs in the reference's own layout (operator tuple
 from the reference's ``get_operators``; parameters under the reference
@@ -25,7 +25,7 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
 
-from ref_import import import_reference  # noqa: E402
+from ref_import import import_reference, reference_src  # noqa: E402
 import diffusion_net_b200.synthetic as syn  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -88,8 +88,15 @@ def run_block(dn, C, params, x, ops, **kw):
     return res
 
 
-def main():
+def main(only=()):
+    """Writes every fixture, or only the files named in `only`.  Every section runs either way: the reference's
+    module constructors draw from the global torch generator, so later fixtures depend on the sections before them."""
     os.makedirs(OUT, exist_ok=True)
+
+    def save(fname, arrays):
+        if not only or fname in only:
+            np.savez_compressed(os.path.join(OUT, fname), **arrays)
+
     dn = import_reference()
     torch.manual_seed(0)
 
@@ -104,7 +111,7 @@ def main():
     fx.update(pack_ops("", mass, evals, evecs, gradX, gradY))
     fx.update({"p:" + k: v.numpy() for k, v in params.items()})
     fx.update(run_block(dn, C, params, x, ops))
-    np.savez_compressed(os.path.join(OUT, "block_small.npz"), **fx)
+    save("block_small.npz", fx)
 
     # ---- 2. no rotations / 3. no gradient features (same operators) ----
     for name, kw in (("block_norot", dict(with_gradient_rotations=False)),
@@ -113,11 +120,12 @@ def main():
         fx2 = {"x_in": x.numpy()}
         fx2.update({"p:" + k: v.numpy() for k, v in p2.items()})
         fx2.update(run_block(dn, C, p2, x, ops, **kw))
-        np.savez_compressed(os.path.join(OUT, name + ".npz"), **fx2)
+        save(name + ".npz", fx2)
 
-    # ---- 4. K=128, C=128 block (human-seg shape at small V) ----
+    # ---- 4. K=128, C=128 block (human-seg widths on a 12x16 torus: V=192, one full 128-row tile and a ragged one;
+    #         the mesh is kept this small so that the fixture stays well under 1 MB) ----
     C4, K4 = 128, 128
-    v4, f4, mass4, L4, evals4, evecs4, gX4, gY4 = ref_operators(dn, 20, 30, K4, seed=3)
+    v4, f4, mass4, L4, evals4, evecs4, gX4, gY4 = ref_operators(dn, 12, 16, K4, seed=3)
     x4 = torch.randn(mass4.shape[0], C4, generator=torch.Generator().manual_seed(11))
     p4 = syn.block_weights(C4, seed=2)
     fx4 = {"x_in": x4.numpy()}
@@ -127,7 +135,7 @@ def main():
     # gold kept fp32-rounded here to keep the fixture small (adds <=6e-8 relative)
     for k in ("x_diffuse_f64", "out_f64"):
         fx4[k + "_as32"] = r4[k].astype(np.float32)
-    np.savez_compressed(os.path.join(OUT, "block_k128.npz"), **fx4)
+    save("block_k128.npz", fx4)
 
     # ---- 5. whole net, 2 blocks, all outputs_at modes, batched B=2 ----
     Cin, Cout, Cw, NB = 3, 8, 32, 2
@@ -160,11 +168,11 @@ def main():
                     ob = nt(st(verts, verts_b), st(mass, mass_b), L=None, evals=st(evals, evals_b),
                             evecs=st(evecs, evecs_b), gradX=st(gradX, gX_b), gradY=st(gradY, gY_b))
                     fxn["out_batch2_" + tag] = ob.numpy()
-    np.savez_compressed(os.path.join(OUT, "net_small.npz"), **fxn)
+    save("net_small.npz", fxn)
 
     # ---- 6. state_dict manifest of the shipped checkpoints (names/shapes only) ----
     man = {}
-    exp = "/root/reference/experiments"
+    exp = os.path.join(os.path.dirname(reference_src()), "experiments")
     for sub, fn in (("human_segmentation_original", "human_seg_xyz_4x128.pth"),
                     ("human_segmentation_original", "human_seg_hks_4x128.pth"),
                     ("functional_correspondence", "faust_xyz.pth"),
@@ -177,11 +185,25 @@ def main():
                 continue
             sdp = torch.load(os.path.join(d, f), map_location="cpu", weights_only=True)
             man[sub + "/" + f] = {k: list(v.shape) for k, v in sdp.items()}
-    with open(os.path.join(OUT, "statedict_manifest.json"), "w") as fh:
-        json.dump(man, fh, indent=1, sort_keys=True)
+    if not only or "statedict_manifest.json" in only:
+        with open(os.path.join(OUT, "statedict_manifest.json"), "w") as fh:
+            json.dump(man, fh, indent=1, sort_keys=True)
+
+    # ---- 7. one shipped checkpoint: every name in file order with its shape, and a seeded sample of 16 values per
+    #         tensor (the whole file is 1.9 MB) ----
+    ckpt = os.path.join(exp, "human_segmentation_original", "pretrained_models", "human_seg_xyz_4x128.pth")
+    if os.path.isfile(ckpt):
+        sdp = torch.load(ckpt, map_location="cpu", weights_only=True)
+        rs = np.random.RandomState(0)
+        fxc = {"names": np.array(list(sdp))}
+        for k, v in sdp.items():
+            flat = v.reshape(-1).numpy()
+            idx = np.sort(rs.choice(flat.size, min(16, flat.size), replace=False)).astype(np.int64)
+            fxc.update({"shape:" + k: np.array(v.shape, dtype=np.int64), "idx:" + k: idx, "val:" + k: flat[idx]})
+        save("checkpoint_human_seg_xyz_4x128.npz", fxc)
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])

@@ -10,7 +10,7 @@ import sys
 import pytest
 import torch
 
-from conftest import ROOT, GOLDEN
+from conftest import ROOT, GOLDEN, load_golden
 
 import diffusion_net_b200 as dn
 
@@ -31,7 +31,8 @@ def test_library_builds_and_exports_header_symbols():
 
 
 def test_sass_is_sm100a_only():
-    out = subprocess.run(["cuobjdump", "-lelf", dn._lib.LIB_PATH], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(dn._lib.nvcc()), "cuobjdump")     # beside nvcc, which need not be on PATH
+    out = subprocess.run([cuobjdump, "-lelf", dn._lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
@@ -54,13 +55,23 @@ def test_state_dict_keys_match_shipped_checkpoints():
 
 
 def test_live_checkpoint_strict_load():
-    path = "/root/reference/experiments/human_segmentation_original/pretrained_models/human_seg_xyz_4x128.pth"
-    if not os.path.exists(path):
-        pytest.skip("reference checkpoints only exist in the build container")
-    sd = torch.load(path, map_location="cpu", weights_only=True)
+    """The reference's pretrained human-segmentation model (human_seg_xyz_4x128.pth), rebuilt from its stored names,
+    order and shapes with a sample of its values (oracle/make_golden.py), loads strictly, and every sampled value lands
+    in the parameter of that name."""
+    fx = load_golden("checkpoint_human_seg_xyz_4x128")
+    names = [str(k) for k in fx["names"]]
+    sd = {}
+    for k in names:
+        t = torch.zeros(tuple(int(s) for s in fx["shape:" + k]))
+        t.view(-1)[torch.from_numpy(fx["idx:" + k])] = torch.from_numpy(fx["val:" + k])
+        sd[k] = t
     net = dn.DiffusionNet(C_in=3, C_out=8, C_width=128, N_block=4, outputs_at="faces")
     net.load_state_dict(sd, strict=True)
     assert len(net.blocks) == 4 and net.blocks[0] is net.block_0
+    ours = net.state_dict()
+    assert list(ours) == names
+    for k in names:
+        assert torch.equal(ours[k].view(-1)[torch.from_numpy(fx["idx:" + k])], torch.from_numpy(fx["val:" + k])), k
 
 
 def test_variant_keys_and_module_layout():
