@@ -95,6 +95,10 @@ SIGNATURES = {
     "dn_from_basis": (_I, [_P, _P, _P, _L, _I, _I, _P, _P, _L, _I, _P]),
     "dn_learned_time_diffusion_fwd": (_I, [_P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P, _L, _I, _P]),
     "dn_learned_time_diffusion_bwd": (_I, [_P, _P, _P, _P, _P, _P, _L, _I, _I, _P, _P, _P, _L, _I, _P]),
+    "dn_learned_time_diffusion_fwd_batched": (_I, [_P, _P, _P, _P, _P, C.POINTER(dn_mesh_batch), _L, _I, _I, _P, _P, _P, _L,
+                                                   _I, _P]),
+    "dn_learned_time_diffusion_bwd_batched": (_I, [_P, _P, _P, _P, _P, _P, C.POINTER(dn_mesh_batch), _L, _I, _I, _P, _P, _P,
+                                                   _L, _I, _P]),
     "dn_grad_spmm": (_I, [C.POINTER(dn_csr), _P, _L, _I, _P, _P]),
     "dn_spatial_gradient_features_fwd": (_I, [_P, _P, _P, _I, _L, _I, _P, _P, _L, _I, _P]),
     "dn_gradient_features_fwd": (_I, [C.POINTER(dn_csr), _P, _P, _P, _I, _L, _I, _P, _P, _P, _L, _I, _P]),

@@ -148,6 +148,43 @@ int one_layer(const DnRowsSrc& src, DnLayer& L, int64_t V, int engine, void* tc_
   return simt_rows_gemm(src, L, V, st);
 }
 
+// grouped split-V to_basis over a mesh batch: every CTA reduces a row range inside one mesh (batch->tb_rows) into its
+// own K x C partial; C_width = 256 runs as two 128-column launches into the same partials
+int grouped_to_basis(const float* values, const float* basis, const float* massvec, int64_t V, int K, int C,
+                     float* partial, const dn_mesh_batch* batch, int engine, cudaStream_t st) {
+  int P = 0;
+  if (tc_to_basis_supported(K, C) == DN_OK)
+    return tc_to_basis_partial(values, basis, massvec, V, K, C, partial, &P, tc_passes(engine), st, 0, 0, batch->tb_rows,
+                               batch->n_tb_ctas);
+  if (!(C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK)) return DN_ERR_UNSUPPORTED;
+  for (int c0 = 0; c0 < C; c0 += 128) {
+    const int rc = tc_to_basis_partial(values + c0, basis, massvec, V, K, 128, partial + c0, &P, tc_passes(engine), st, C,
+                                       C, batch->tb_rows, batch->n_tb_ctas);
+    if (rc) return rc;
+  }
+  return DN_OK;
+}
+
+// Support checks of the grouped spectral stage (learned-time diffusion over a mesh batch), all made before anything is
+// enqueued: the grouped to_basis, and a from_basis chain `L` that picks its weights per tile.  Chooses L's pack format.
+int grouped_spectral_check(const float* values, const float* evecs, const dn_mesh_batch* batch, int64_t V, int K, int C,
+                           int engine, DnLayer* L) {
+  if (!batch || batch->n_meshes < 1 || batch->n_tb_ctas < 1 || !batch->tile_mesh || !batch->tb_rows ||
+      !batch->mesh_cta_begin)
+    return DN_ERR_INVALID_ARGUMENT;
+  if (!use_tc(engine)) return DN_ERR_UNSUPPORTED;
+  if (!tc_supported_device()) return DN_ERR_NOT_SM100;
+  if ((V % 128) || V >= (1ll << 31) - 256 || (C % 4) || (reinterpret_cast<uintptr_t>(values) & 15) ||
+      (reinterpret_cast<uintptr_t>(evecs) & 15))
+    return DN_ERR_UNSUPPORTED;
+  if (tc_to_basis_supported(K, C) != DN_OK && !(C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK))
+    return DN_ERR_UNSUPPORTED;
+  const DnRowsSrc src = one_src(evecs, K, K);
+  if (tc_grouped_chain_supported(src, L, 1, tc_passes(engine)) != DN_OK) return DN_ERR_UNSUPPORTED;
+  tc_choose_pack_fmt(src, L, 1, tc_passes(engine));
+  return DN_OK;
+}
+
 }  // namespace
 
 long long g_dn_launches = 0;
@@ -375,6 +412,56 @@ int dn_learned_time_diffusion_bwd(const float* grad_out, const float* mass, cons
   DnLayer L = make_layer(dS, C, 1, nullptr, 0, K, C, grad_x, C);
   L.row_scale = mass;
   return run_chain(src, &L, 1, V, engine, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st);
+}
+
+int dn_learned_time_diffusion_fwd_batched(const float* x, const float* mass, const float* evals, const float* evecs,
+                                          float* time, const dn_mesh_batch* batch, int64_t V, int K, int C,
+                                          float* x_diffuse, float* x_spec_out, void* workspace, int64_t ws_bytes,
+                                          int engine, dn_stream_t stream) {
+  if (!x || !mass || !evals || !evecs || !time || !x_diffuse || V < 0 || K <= 0 || C <= 0)
+    return DN_ERR_INVALID_ARGUMENT;
+  DnLayer L = make_layer(nullptr, C, /*w_trans=*/1, nullptr, 0, K, C, x_diffuse, C);
+  int rc = grouped_spectral_check(x, evecs, batch, V, K, C, engine, &L);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  Bump ws(workspace, ws_bytes);
+  const int64_t pb = tc_chain_ws_bytes(&L, 1) * batch->n_meshes;
+  float* pk = ws.take(pb / 4);
+  float* partial = ws.take((int64_t)batch->n_tb_ctas * K * C);
+  if (!pk || !partial) return DN_ERR_WORKSPACE;
+  // (nothing has been enqueued up to here)
+  if ((rc = grouped_to_basis(x, evecs, mass, V, K, C, partial, batch, engine, st))) return rc;
+  if ((rc = tc_pack_spectral_batched(&L, batch->n_meshes, pk, pb, partial, batch->mesh_cta_begin, evals, time,
+                                     /*clamp_writeback=*/1, batch->tile_mesh, st, x_spec_out)))
+    return rc;
+  return tc_rows_chain(one_src(evecs, K, K), &L, 1, V, tc_passes(engine), ws.base + ws.off, ws.size - ws.off, st);
+}
+
+int dn_learned_time_diffusion_bwd_batched(const float* grad_out, const float* mass, const float* evals,
+                                          const float* evecs, const float* time, const float* x_spec,
+                                          const dn_mesh_batch* batch, int64_t V, int K, int C, float* grad_x,
+                                          float* grad_time, void* workspace, int64_t ws_bytes, int engine,
+                                          dn_stream_t stream) {
+  if (!grad_out || !mass || !evals || !evecs || !time || !x_spec || !grad_x || !grad_time || V < 0 || K <= 0 || C <= 0)
+    return DN_ERR_INVALID_ARGUMENT;
+  // grad_x = mass * (Phi_b dS_b) per tile: the from_basis chain with per-mesh weights and a row_scale epilogue
+  DnLayer L = make_layer(nullptr, C, /*w_trans=*/1, nullptr, 0, K, C, grad_x, C);
+  L.row_scale = mass;
+  int rc = grouped_spectral_check(grad_out, evecs, batch, V, K, C, engine, &L);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  Bump ws(workspace, ws_bytes);
+  const int64_t pb = tc_chain_ws_bytes(&L, 1) * batch->n_meshes;
+  float* pk = ws.take(pb / 4);
+  float* dt = ws.take(tc_spectral_bwd_batched_scratch_floats(batch->n_meshes, K, C));
+  float* partial = ws.take((int64_t)batch->n_tb_ctas * K * C);
+  if (!pk || !dt || !partial) return DN_ERR_WORKSPACE;
+  // (nothing has been enqueued up to here)
+  if ((rc = grouped_to_basis(grad_out, evecs, nullptr, V, K, C, partial, batch, engine, st))) return rc;
+  if ((rc = tc_spectral_bwd_batched(&L, batch->n_meshes, pk, pb, partial, batch->mesh_cta_begin, evals, time, x_spec, dt,
+                                    grad_time, batch->tile_mesh, st)))
+    return rc;
+  return tc_rows_chain(one_src(evecs, K, K), &L, 1, V, tc_passes(engine), ws.base + ws.off, ws.size - ws.off, st);
 }
 
 int dn_grad_spmm(const dn_csr* grad, const float* x, int64_t V, int C, float* out, dn_stream_t stream) {
@@ -714,18 +801,7 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
     if (!use_tc(engine) || !tc_supported_device() || (V % 128) || batch->n_meshes < 1 || !batch->tile_mesh ||
         !batch->tb_rows || !batch->mesh_cta_begin || batch->n_tb_ctas < 1 || (int64_t)batch->n_tb_ctas * K * C > pf)
       return DN_ERR_UNSUPPORTED;
-    if (tc_to_basis_supported(K, C) == DN_OK) {
-      if ((rc = tc_to_basis_partial(x_in, evecs, mass, V, K, C, partial, &P, tc_passes(engine), st, 0, 0, batch->tb_rows,
-                                    batch->n_tb_ctas)))
-        return rc;
-    } else if (C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK) {
-      for (int c0 = 0; c0 < C; c0 += 128)
-        if ((rc = tc_to_basis_partial(x_in + c0, evecs, mass, V, K, 128, partial + c0, &P, tc_passes(engine), st, C, C,
-                                      batch->tb_rows, batch->n_tb_ctas)))
-          return rc;
-    } else {
-      return DN_ERR_UNSUPPORTED;
-    }
+    if ((rc = grouped_to_basis(x_in, evecs, mass, V, K, C, partial, batch, engine, st))) return rc;
   } else if ((rc = to_basis_partials(x_in, evecs, mass, V, K, C, partial, pf, &P, engine, st))) {
     return rc;
   }

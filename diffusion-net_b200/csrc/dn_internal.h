@@ -149,10 +149,21 @@ int tc_to_basis_partial(const float* values, const float* basis, const float* ma
 int tc_to_basis_supported(int K, int C);
 int64_t tc_chain_ws_bytes(const DnLayer* layers, int n_layers);
 // mesh batches: pack S_b = exp(-evals_b t) * (partials of mesh b) for every mesh as layer0's per-mesh weights
-// (ws: n_meshes * tc_chain_ws_bytes(layer0, 1) bytes); sets layer0->prepacked / tile_group / group_stride
+// (ws: n_meshes * tc_chain_ws_bytes(layer0, 1) bytes); sets layer0->prepacked / tile_group / group_stride.
+// x_spec_out (optional, [n_meshes][K][N]) receives every mesh's reduced, unscaled coefficients.
 int tc_pack_spectral_batched(DnLayer* layer0, int n_meshes, void* ws, int64_t ws_bytes, const float* partial,
                              const int32_t* mesh_cta_begin, const float* evals, float* time, int clamp_writeback,
-                             const int32_t* tile_mesh, cudaStream_t st);
+                             const int32_t* tile_mesh, cudaStream_t st, float* x_spec_out = nullptr);
+// mesh batches, backward (two launches): from the partials of Phi_b^T g_b, pack dS_b = exp(-evals_b t) * Gs_b as layer0's
+// per-mesh weights (as above) and add sum_b sum_k Gs_b * (-lambda_bk) * E_b * x_spec_b to grad_time in a fixed order.
+// dt_scratch: tc_spectral_bwd_batched_scratch_floats(n_meshes, K, N) floats.
+#define DN_SPEC_BWD_KROWS 4
+int64_t tc_spectral_bwd_batched_scratch_floats(int n_meshes, int K, int N);
+int tc_spectral_bwd_batched(DnLayer* layer0, int n_meshes, void* ws, int64_t ws_bytes, const float* partial,
+                            const int32_t* mesh_cta_begin, const float* evals, const float* time, const float* x_spec,
+                            float* dt_scratch, float* grad_time, const int32_t* tile_mesh, cudaStream_t st);
+// the chain kernels that can pick layer-0 weights per tile (tile_group): chain3, and chain16 on the bf16 engine
+int tc_grouped_chain_supported(const DnRowsSrc& src, const DnLayer* layers, int n_layers, int passes);
 // one launch: pack the weights of n layers into ws and set layers[i].prepacked
 int tc_pack_layers(DnLayer* layers, int n_layers, void* ws, int64_t ws_bytes, cudaStream_t st);
 // same, with layers[0] (w_trans, K = eigen count, N = channels) replaced by the spectral multiplier

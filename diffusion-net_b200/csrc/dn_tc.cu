@@ -167,10 +167,11 @@ __global__ void pack_weights_kernel(const __grid_constant__ PackJobs jobs) {
 
 // mesh batches: the spectral multiplier of every mesh, packed as layer-0 weights of the from_basis chain
 //   S_b[k][n] = exp(-evals[b][k] * max(t[n], 1e-8)) * sum_{p in CTAs of mesh b} partial[p][k][n]     (layers.py:48-49, 62-64)
-// grid (ceil(K*N/32), n_meshes), 256 threads: 32 consecutive elements x 8 slices of the partial sums per block
+// grid (ceil(K*N/32), n_meshes), 256 threads: 32 consecutive elements x 8 slices of the partial sums per block.
+// x_spec_out (optional, [n_meshes][K][N]): the reduced, unscaled coefficients of every mesh (saved for the backward pass)
 __global__ void spectral_pack_batched_kernel(const float* __restrict__ partial, const int32_t* __restrict__ mesh_cta_begin,
                                              const float* __restrict__ evals, float* time, int K, int N, int fmt, int kc,
-                                             float* dst, int64_t dst_stride_floats, int clamp) {
+                                             float* dst, int64_t dst_stride_floats, int clamp, float* __restrict__ x_spec_out) {
   __shared__ float red[8][33];
   const int b = blockIdx.y;
   const int e = threadIdx.x & 31, sl = threadIdx.x >> 5;
@@ -190,9 +191,67 @@ __global__ void spectral_pack_batched_kernel(const float* __restrict__ partial, 
   const float t = fmaxf(time[n], 1e-8f);
   const float w = expf(-(evals[(int64_t)b * K + k] * t)) * sum;
   pack_store(dst + (int64_t)b * dst_stride_floats, fmt, kc, N, k, n, w);
+  if (x_spec_out) x_spec_out[(int64_t)b * K * N + idx] = sum;
   // the in-place clamp of the reference: written back by mesh 0 only, after every reader of t[n] in this launch has at
   // worst read either value (max(t, 1e-8) is idempotent)
   if (clamp && b == 0 && k == K - 1) time[n] = t;
+}
+
+// mesh batches, backward of the spectral multiplier (the batched form of spectral_bwd_kernel):
+//   Gs_b[k][n] = sum_{p in CTAs of mesh b} partial[p][k][n]   (= Phi_b^T g_b),
+//   dS_b = exp(-evals[b][k] t[n]) * Gs_b   packed as mesh b's layer-0 weights of the from_basis chain,
+//   dt_part[b * gridDim.y + kg][n] = sum over the DN_SPEC_BWD_KROWS rows k of group kg of Gs_b * (-lambda) * E * x_spec_b.
+// grid (ceil(N/32), ceil(K/DN_SPEC_BWD_KROWS), n_meshes), 256 threads: 32 consecutive columns x 8 slices of the partials.
+// Every sum runs in a fixed order (no atomics): the result does not depend on scheduling.
+__global__ void spectral_bwd_pack_batched_kernel(const float* __restrict__ partial, const int32_t* __restrict__ mesh_cta_begin,
+                                                 const float* __restrict__ evals, const float* __restrict__ time,
+                                                 const float* __restrict__ x_spec, int K, int N, int fmt, int kc, float* dst,
+                                                 int64_t dst_stride_floats, float* __restrict__ dt_part) {
+  __shared__ float red[8][33];
+  const int b = blockIdx.z, kg = blockIdx.y;
+  const int e = threadIdx.x & 31, sl = threadIdx.x >> 5;
+  const int n = (int)blockIdx.x * 32 + e;
+  const int p0 = mesh_cta_begin[b], p1 = mesh_cta_begin[b + 1];
+  const int64_t stride = (int64_t)K * N;
+  const float t = n < N ? fmaxf(time[n], 1e-8f) : 0.f;
+  float dt = 0.f;
+  for (int i = 0; i < DN_SPEC_BWD_KROWS; ++i) {
+    const int k = kg * DN_SPEC_BWD_KROWS + i;
+    const bool live = k < K && n < N;
+    float acc = 0.f;
+    if (live) {
+      const float* pp = partial + (int64_t)k * N + n;
+      for (int q = p0 + sl; q < p1; q += 8) acc += pp[(int64_t)q * stride];
+    }
+    red[sl][e] = acc;
+    __syncthreads();
+    if (sl == 0 && live) {
+      const float g = ((red[0][e] + red[1][e]) + (red[2][e] + red[3][e])) + ((red[4][e] + red[5][e]) + (red[6][e] + red[7][e]));
+      const float lam = evals[(int64_t)b * K + k];
+      const float ex = expf(-(lam * t));
+      pack_store(dst + (int64_t)b * dst_stride_floats, fmt, kc, N, k, n, ex * g);
+      dt += g * (-lam) * ex * x_spec[(int64_t)b * stride + (int64_t)k * N + n];
+    }
+    __syncthreads();
+  }
+  if (sl == 0 && n < N) dt_part[((int64_t)b * gridDim.y + kg) * N + n] = dt;
+}
+
+// grad_time[n] += sum_r dt_part[r][n] in a fixed order.  grid ceil(N/32), 1024 threads: 32 columns x 32 row slices
+__global__ void grad_time_reduce_kernel(const float* __restrict__ dt_part, int rows, int N, float* __restrict__ grad_time) {
+  __shared__ float red[32][33];
+  const int e = threadIdx.x & 31, sl = threadIdx.x >> 5;
+  const int n = (int)blockIdx.x * 32 + e;
+  float s = 0.f;
+  if (n < N)
+    for (int r = sl; r < rows; r += 32) s += dt_part[(int64_t)r * N + n];
+  red[sl][e] = s;
+  __syncthreads();
+  if (sl != 0 || n >= N) return;
+  float tot = 0.f;
+#pragma unroll
+  for (int i = 0; i < 32; ++i) tot += red[i][e];
+  grad_time[n] += tot;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1252,7 +1311,7 @@ int tc_pack_layers_spectral(DnLayer* layers, int n_layers, void* ws, int64_t ws_
 
 int tc_pack_spectral_batched(DnLayer* layer0, int n_meshes, void* ws, int64_t ws_bytes, const float* partial,
                              const int32_t* mesh_cta_begin, const float* evals, float* time, int clamp_writeback,
-                             const int32_t* tile_mesh, cudaStream_t st) {
+                             const int32_t* tile_mesh, cudaStream_t st, float* x_spec_out) {
   if (!layer0 || n_meshes < 1 || !ws || !partial || !mesh_cta_begin || !evals || !time || !tile_mesh)
     return DN_ERR_INVALID_ARGUMENT;
   const int64_t per = tc_chain_ws_bytes(layer0, 1);
@@ -1260,12 +1319,43 @@ int tc_pack_spectral_batched(DnLayer* layer0, int n_meshes, void* ws, int64_t ws
   const int K = layer0->K, N = layer0->N;
   dim3 grid((unsigned)((K * N + 31) / 32), (unsigned)n_meshes);
   spectral_pack_batched_kernel<<<grid, 256, 0, st>>>(partial, mesh_cta_begin, evals, time, K, N, layer0->pack_fmt, KC,
-                                                     static_cast<float*>(ws), per / 4, clamp_writeback);
+                                                     static_cast<float*>(ws), per / 4, clamp_writeback, x_spec_out);
   DN_LAUNCH_CHECK();
   layer0->prepacked = static_cast<float*>(ws);
   layer0->tile_group = tile_mesh;
   layer0->group_stride = per / 4;
   return DN_OK;
+}
+
+int64_t tc_spectral_bwd_batched_scratch_floats(int n_meshes, int K, int N) {
+  return (int64_t)n_meshes * ((K + DN_SPEC_BWD_KROWS - 1) / DN_SPEC_BWD_KROWS) * N;
+}
+
+int tc_spectral_bwd_batched(DnLayer* layer0, int n_meshes, void* ws, int64_t ws_bytes, const float* partial,
+                            const int32_t* mesh_cta_begin, const float* evals, const float* time, const float* x_spec,
+                            float* dt_scratch, float* grad_time, const int32_t* tile_mesh, cudaStream_t st) {
+  if (!layer0 || n_meshes < 1 || !ws || !partial || !mesh_cta_begin || !evals || !time || !x_spec || !dt_scratch ||
+      !grad_time || !tile_mesh)
+    return DN_ERR_INVALID_ARGUMENT;
+  const int64_t per = tc_chain_ws_bytes(layer0, 1);
+  if (per * n_meshes > ws_bytes) return DN_ERR_WORKSPACE;
+  const int K = layer0->K, N = layer0->N;
+  const int kgroups = (K + DN_SPEC_BWD_KROWS - 1) / DN_SPEC_BWD_KROWS;
+  dim3 grid((unsigned)((N + 31) / 32), (unsigned)kgroups, (unsigned)n_meshes);
+  spectral_bwd_pack_batched_kernel<<<grid, 256, 0, st>>>(partial, mesh_cta_begin, evals, time, x_spec, K, N,
+                                                         layer0->pack_fmt, KC, static_cast<float*>(ws), per / 4, dt_scratch);
+  DN_LAUNCH_CHECK();
+  grad_time_reduce_kernel<<<(N + 31) / 32, 1024, 0, st>>>(dt_scratch, n_meshes * kgroups, N, grad_time);
+  DN_LAUNCH_CHECK();
+  layer0->prepacked = static_cast<float*>(ws);
+  layer0->tile_group = tile_mesh;
+  layer0->group_stride = per / 4;
+  return DN_OK;
+}
+
+int tc_grouped_chain_supported(const DnRowsSrc& src, const DnLayer* layers, int n_layers, int passes) {
+  if (passes == DN_PASSES_BF16 && tc_chain16_supported(src, layers, n_layers) == DN_OK) return DN_OK;
+  return tc_chain3_supported(src, layers, n_layers);
 }
 
 int tc_rows_chain(const DnRowsSrc& src, const DnLayer* layers_in, int n_layers, int64_t V, int passes, void* ws,

@@ -97,7 +97,8 @@ class GraphedBatch:
 
 
 class GraphedTrainStep:
-    """Forward + backward of ``loss_fn(net, *inputs)`` for one fixed set of input tensors (one mesh) as ONE CUDA graph.
+    """Forward + backward of ``loss_fn(net, *inputs)`` for one fixed set of input tensors (one mesh, or a whole
+    ``batch.MeshBatch`` when ``loss_fn`` calls ``net.forward_batch``) as ONE CUDA graph.
 
     A 4-block DiffusionNet training step on a human-seg-sized mesh is ~190 launches of 5-20 us each: eager autograd is
     launch-bound (BASELINE configs 2 and 5).  The graph is captured once per mesh (PyTorch's whole-network capture

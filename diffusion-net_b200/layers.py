@@ -197,6 +197,19 @@ class DiffusionNetBlock(nn.Module):
         outs = [self._forward_mesh(x_in[b], mass[b], evals[b], evecs[b], gops[b], fused, head) for b in range(B)]
         return torch.stack(outs, dim=0)
 
+    def forward_batch(self, batch, x_in):
+        """Differentiable block over every mesh of a ``batch.MeshBatch`` (``x_in``: (batch.V, C_width) in the batch
+        layout): batched spectral diffusion, the gradient features on the block-diagonal CSR and the MiniMLP, each one
+        launch sequence over all meshes.  Training-mode dropout applies (MiniMLP masks)."""
+        if self.diffusion.method != 'spectral':
+            raise NotImplementedError("forward_batch: spectral diffusion only")
+        x_diffuse = ops.batched_diffusion(x_in, self.diffusion.diffusion_time, batch)
+        srcs = [x_in, x_diffuse]
+        if self.with_gradient_features:
+            A_re, A_im = self.gradient_features.weights()
+            srcs.append(ops.GradFeaturesFn.apply(x_diffuse, A_re, A_im, batch.gops))
+        return self.mlp.forward_sources(srcs, residual=x_in)   # layers.py:229-239
+
 
 class DiffusionNet(nn.Module):
 
@@ -238,29 +251,62 @@ class DiffusionNet(nn.Module):
         B = x.shape[0]
         return torch.stack([ops.mlp_apply([x[b]], [lin.weight], [lin.bias]) for b in range(B)], 0)
 
-    def forward_batch(self, batch, xs):
-        """Inference over a ``batch.MeshBatch`` of independent meshes in ONE launch sequence (BASELINE config 4): the
-        reference's per-mesh loop (layers.py:217-222, 366-401) with every stage of every block launched once over all
-        meshes (``dn_block_fwd_batched``).  ``xs``: list of per-mesh (V_b, C_in) features, or one tensor already in the
-        batch layout.  Returns the list of per-mesh outputs (views into one tensor); 'vertices' and 'global_mean'
-        outputs only.  Equal to ``[self(x_b, mass_b, ...) for b]`` (tests/test_gpu_parity.py)."""
-        from . import batch as _batch
-        if self.outputs_at not in ('vertices', 'global_mean'):
-            raise ValueError("forward_batch supports outputs_at 'vertices' and 'global_mean'")
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-            raise RuntimeError("forward_batch is an inference path: call it under torch.no_grad()")
+    def forward_batch(self, batch, xs, edges=None, faces=None):
+        """The network over a ``batch.MeshBatch`` of independent meshes in ONE launch sequence (BASELINE configs 4 and
+        5): the reference's per-mesh loop (layers.py:217-222, 366-401) with every stage of every block launched once over
+        all meshes.  ``xs``: list of per-mesh (V_b, C_in) features, or one tensor already in the batch layout.
+        ``edges`` / ``faces``: lists of per-mesh (E_b, 2) / (F_b, 3) vertex indices local to each mesh, for
+        ``outputs_at`` 'edges' / 'faces'.  Returns the list of per-mesh outputs.  Equal to ``[self(x_b, mass_b, ...) for
+        b]`` (tests/test_gpu_parity.py, tests/test_gpu_batch_train.py).
+
+        Under ``torch.no_grad()`` (or with nothing to differentiate) this is the fused inference route
+        (``dn_block_fwd_batched``, last_lin fused when possible).  With autograd on it is differentiable: first_lin ->
+        per block ``DiffusionNetBlock.forward_batch`` -> last_lin over the whole range, so a training step over any
+        number of meshes is one fixed launch sequence (and can be captured as one graph, graphs.GraphedTrainStep)."""
         if self.diffusion_method != 'spectral':
             raise NotImplementedError("forward_batch: spectral diffusion only")
+        elems = None
+        if self.outputs_at in ('edges', 'faces'):
+            elems = edges if self.outputs_at == 'edges' else faces
+            if elems is None or len(elems) != batch.n_meshes:
+                raise ValueError("forward_batch with outputs_at='{}' needs one index tensor per mesh in `{}`".format(
+                    self.outputs_at, self.outputs_at))
         x = xs if torch.is_tensor(xs) else batch.pack(xs)
         if x.shape[-1] != self.C_in:
             raise ValueError("DiffusionNet was constructed with C_in={}, but x_in has last dim={}".format(
                 self.C_in, x.shape[-1]))
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+            _ = batch.gops.csr_t           # the gather's backward needs the transposed CSR: build it now, not mid-capture
+            x = ops.mlp_apply([x], [self.first_lin.weight], [self.first_lin.bias])
+            for blk in self.blocks:
+                x = blk.forward_batch(batch, x)
+            x = ops.mlp_apply([x], [self.last_lin.weight], [self.last_lin.bias])
+        else:
+            x = self._forward_batch_fused(batch, x)
+        outs = batch.unpack(x)
+        if elems is not None:
+            # mean of the per-vertex outputs over each element's corners, as ``forward`` does
+            outs = [o[e].mean(dim=1) for o, e in zip(outs, elems)]
+        elif self.outputs_at == 'global_mean':
+            res = []
+            for b, o in enumerate(outs):
+                m = batch.mass[batch.row_begin[b]:batch.row_begin[b] + batch.n_rows[b]]
+                res.append((o * (m / m.sum()).unsqueeze(-1)).sum(dim=-2))
+            outs = res
+        if self.last_activation != None:
+            outs = [self.last_activation(o) for o in outs]
+        return outs
+
+    def _forward_batch_fused(self, batch, x):
+        """Inference route of ``forward_batch``: batch-layout input -> per-vertex outputs (V, C_out), batch layout."""
+        from . import batch as _batch
         x = ops.mlp_apply([x], [self.first_lin.weight], [self.first_lin.bias])
         fuse_head = FUSE_HEAD and ops.head_fusable(self.C_out)
         head_done = False
         for i_b, blk in enumerate(self.blocks):
             if blk.training and blk.dropout:
-                raise RuntimeError("forward_batch: eval mode only (dropout)")
+                raise RuntimeError("forward_batch under no_grad: eval mode only (dropout); training-mode dropout runs "
+                                   "with autograd on")
             A_re = A_im = None
             if blk.with_gradient_features:
                 A_re, A_im = blk.gradient_features.weights()
@@ -277,16 +323,7 @@ class DiffusionNet(nn.Module):
             x = _batch.block_forward_batched_raw(*args)
         if not head_done:
             x = ops.mlp_apply([x], [self.last_lin.weight], [self.last_lin.bias])
-        outs = batch.unpack(x)
-        if self.outputs_at == 'global_mean':
-            res = []
-            for b, o in enumerate(outs):
-                m = batch.mass[batch.row_begin[b]:batch.row_begin[b] + batch.n_rows[b]]
-                res.append((o * (m / m.sum()).unsqueeze(-1)).sum(dim=-2))
-            outs = res
-        if self.last_activation != None:
-            outs = [self.last_activation(o) for o in outs]
-        return outs
+        return x
 
     def forward(self, x_in, mass, L=None, evals=None, evecs=None, gradX=None, gradY=None, edges=None, faces=None):
         """[N,C] or [B,N,C] in, [N,C_out] or [B,N,C_out] out (reference layers.py:314-407)."""

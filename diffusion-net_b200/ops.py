@@ -595,6 +595,85 @@ class DiffusionFn(torch.autograd.Function):
         return gx, gt, None, None, None
 
 
+class _BatchUnsupported(Exception):
+    """dn_learned_time_diffusion_*_batched refused the shape / engine (DN_ERR_UNSUPPORTED, nothing enqueued)."""
+
+
+def _batched_ws(batch, K, Cc, device):
+    # per-mesh packed multipliers (2 K C floats each) + the backward's per-mesh grad_time partials (K C / 4 floats each)
+    return workspace(batch.V, K, Cc, device, extra=int(batch.n_meshes) * K * Cc * 12)
+
+
+class BatchedDiffusionFn(torch.autograd.Function):
+    """layers.py:44-67 spectral LearnedTimeDiffusion over every mesh of a ``batch.MeshBatch`` (``x`` in the batch layout):
+    grouped to_basis, one packed multiplier per mesh and a from_basis chain that picks its weights per tile, forward and
+    backward each a fixed launch sequence whatever the number of meshes (dn_learned_time_diffusion_{fwd,bwd}_batched).
+    Use ``batched_diffusion``, which takes the per-mesh route where these kernels do not apply."""
+
+    @staticmethod
+    @_device_guard
+    def forward(ctx, x, time, batch):
+        lib = _lib.load()
+        x = _f32c(x)
+        V, Cc = x.shape
+        K = batch.K
+        B = batch.n_meshes
+        xd = torch.empty_like(x)
+        x_spec = torch.empty(B, K, Cc, dtype=torch.float32, device=x.device)
+        ws = _batched_ws(batch, K, Cc, x.device)
+        # the kernel clamps `time` in place, as the reference does on the Parameter (layers.py:48-49)
+        rc = lib.dn_learned_time_diffusion_fwd_batched(x.data_ptr(), batch.mass.data_ptr(), batch.evals.data_ptr(),
+                                                       batch.evecs.data_ptr(), time.data_ptr(), C.byref(batch.desc), V, K,
+                                                       Cc, xd.data_ptr(), x_spec.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                       _engine, _stream())
+        if rc == -2:                    # DN_ERR_UNSUPPORTED
+            raise _BatchUnsupported()
+        _lib.check(rc, "dn_learned_time_diffusion_fwd_batched")
+        ctx.batch = batch
+        ctx.save_for_backward(time.detach().clone(), x_spec)
+        return xd
+
+    @staticmethod
+    @_device_guard
+    def backward(ctx, g):
+        lib = _lib.load()
+        time, x_spec = ctx.saved_tensors
+        batch = ctx.batch
+        g = _f32c(g)
+        V, Cc = g.shape
+        K = batch.K
+        gx = torch.empty_like(g)
+        gt = torch.zeros_like(time)
+        ws = _batched_ws(batch, K, Cc, g.device)
+        _lib.check(lib.dn_learned_time_diffusion_bwd_batched(g.data_ptr(), batch.mass.data_ptr(), batch.evals.data_ptr(),
+                                                             batch.evecs.data_ptr(), time.data_ptr(), x_spec.data_ptr(),
+                                                             C.byref(batch.desc), V, K, Cc, gx.data_ptr(), gt.data_ptr(),
+                                                             ws.data_ptr(), ws.numel(), _engine, _stream()),
+                   "dn_learned_time_diffusion_bwd_batched")
+        return gx, gt, None
+
+
+def batched_diffusion(x, time, batch):
+    """Differentiable learned-time diffusion over a mesh batch (``x``: (batch.V, C) in the batch layout).  Shapes and
+    engines outside the grouped kernels (the SIMT engine, K not a multiple of 64, ...) run ``DiffusionFn`` on each mesh's
+    rows instead; padding rows are zero either way."""
+    _require_cuda(x, time)
+    if x.shape[0] != batch.V:
+        raise ValueError("x is not in this batch's layout ({} rows, expected {})".format(x.shape[0], batch.V))
+    try:
+        return BatchedDiffusionFn.apply(x, time, batch)
+    except _BatchUnsupported:
+        pass
+    pieces = []
+    for b in range(batch.n_meshes):
+        r0, n = batch.row_begin[b], batch.n_rows[b]
+        pieces.append(DiffusionFn.apply(x[r0:r0 + n], time, batch.mass[r0:r0 + n], batch.evals[b], batch.evecs[r0:r0 + n]))
+        pad = batch.row_begin[b + 1] - r0 - n
+        if pad:
+            pieces.append(x.new_zeros(pad, x.shape[1]))
+    return torch.cat(pieces, dim=0)
+
+
 class GradFeaturesFn(torch.autograd.Function):
     """layers.py:216-226: sparse tangent gradient + SpatialGradientFeatures, fused."""
 

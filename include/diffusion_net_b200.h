@@ -264,6 +264,26 @@ int dn_block_fwd_batched(const float* x_in, const float* mass, const float* eval
                          const dn_csr* grad, const dn_block_params* params, const dn_mesh_batch* batch, int64_t V,
                          int K, int C, float* out, void* workspace, int64_t ws_bytes, int engine, dn_stream_t stream);
 
+/* layers.py:44-67 LearnedTimeDiffusion over every mesh of a batch laid out as above, differentiable: the training
+ * counterpart of the spectral stage of dn_block_fwd_batched.  evals is (n_meshes, K); time (C) is clamped in place
+ * (layers.py:48-49).  x_spec_out (n_meshes, K, C) optional: mesh b's un-scaled spectral coefficients, saved for the
+ * backward pass.  The launch count does not depend on the number of meshes.  Tensor-core engines only, and only shapes
+ * whose from_basis chain picks its weights per tile: DN_ERR_UNSUPPORTED otherwise (the SIMT engine, K = 32, ...), with
+ * nothing enqueued (the caller then loops over the meshes with dn_learned_time_diffusion_fwd). */
+int dn_learned_time_diffusion_fwd_batched(const float* x, const float* mass, const float* evals, const float* evecs,
+                                          float* time, const dn_mesh_batch* batch, int64_t V, int K, int C,
+                                          float* x_diffuse, float* x_spec_out, void* workspace, int64_t ws_bytes,
+                                          int engine, dn_stream_t stream);
+
+/* Backward of the above w.r.t. x and time; x_spec is what the forward wrote to x_spec_out.  grad_x is written (exactly 0
+ * on padding rows); grad_time (C) is ACCUMULATED into (+=), summed over the meshes in a fixed order (bit-reproducible).
+ * Same support rules as the forward. */
+int dn_learned_time_diffusion_bwd_batched(const float* grad_out, const float* mass, const float* evals,
+                                          const float* evecs, const float* time, const float* x_spec,
+                                          const dn_mesh_batch* batch, int64_t V, int K, int C, float* grad_x,
+                                          float* grad_time, void* workspace, int64_t ws_bytes, int engine,
+                                          dn_stream_t stream);
+
 /* Linear head fused behind a block (SURVEY.md 8f-1): `DiffusionNet.last_lin` (layers.py:366-370 -- the nn.Linear applied
  * to the last block's output) computed in the epilogue of that block's MiniMLP chain, in exact fp32, so that the
  * C_width-wide block output is never written: out_head[v][o] = bias[o] + sum_c weight[o][c] * block_out[v][c]. */
