@@ -24,13 +24,17 @@ struct Bump {
 
 constexpr int64_t kPartialFloats = 16ll << 20;  // 64 MiB split-V partial sums
 
-inline bool use_tc(int engine) { return engine == DN_ENGINE_TC3X || engine == DN_ENGINE_TC1X || engine == DN_ENGINE_BF16; }
-inline int tc_passes(int engine) { return engine == DN_ENGINE_TC1X ? 1 : (engine == DN_ENGINE_BF16 ? DN_PASSES_BF16 : 3); }
+// The engine as the helpers below take it, resolved once per entry point before anything is enqueued: 0 runs the exact
+// fp32 SIMT kernels, otherwise the tensor-core pass count (3, 1 or DN_PASSES_BF16).  A tensor-core engine on a device
+// without tcgen05 is DN_ERR_NOT_SM100: there is no multi-backend dispatch.
+int resolve_engine(int engine, int* tc) {
+  *tc = engine == DN_ENGINE_TC3X ? 3 : engine == DN_ENGINE_TC1X ? 1 : engine == DN_ENGINE_BF16 ? DN_PASSES_BF16 : 0;
+  return (*tc && !tc_supported_device()) ? DN_ERR_NOT_SM100 : DN_OK;
+}
 
 // A tensor-core engine was requested but this contraction is outside the tcgen05 kernels' envelope and runs the exact
 // fp32 SIMT kernel instead (same result class or better, slower).  Said once per shape on stderr; DN_STRICT_TC=1 turns
-// it into DN_ERR_UNSUPPORTED so that a deployment never runs the slow path unnoticed.  A non-sm_100 device with a
-// tensor-core engine is always an error (DN_ERR_NOT_SM100): there is no multi-backend dispatch.
+// it into DN_ERR_UNSUPPORTED so that a deployment never runs the slow path unnoticed.
 int note_simt_fallback(const char* what, int K, int N) {
   static int strict = -1;
   if (strict < 0) { const char* e = getenv("DN_STRICT_TC"); strict = (e && atoi(e)) ? 1 : 0; }
@@ -45,10 +49,6 @@ int note_simt_fallback(const char* what, int K, int N) {
   }
   return strict ? DN_ERR_UNSUPPORTED : DN_OK;
 }
-#define DN_TC_DEVICE_OR_FAIL(engine)                                              \
-  do {                                                                            \
-    if (use_tc(engine) && !tc_supported_device()) return DN_ERR_NOT_SM100;        \
-  } while (0)
 
 inline DnLayer make_layer(const float* W, int64_t ldw, int w_trans, const float* bias, int relu, int K, int N,
                           float* out, int64_t ld_out) {
@@ -66,15 +66,12 @@ inline DnRowsSrc one_src(const float* p, int width, int64_t ld) {
   return s;
 }
 
-// run a chain of layers; tensor-core engine when it supports the shapes, exact SIMT otherwise.
+// run a chain of layers; tensor-core engine `tc` (resolve_engine) when it supports the shapes, exact SIMT otherwise.
 // `tmp0/tmp1` are V x maxN ping-pong buffers used only by the unfused SIMT route.
-int run_chain(const DnRowsSrc& src, DnLayer* layers, int n_layers, int64_t V, int engine, float* tmp0,
-              float* tmp1, void* tc_ws, int64_t tc_ws_bytes, cudaStream_t st) {
-  DN_TC_DEVICE_OR_FAIL(engine);
-  const bool tc = use_tc(engine) && tc_supported_device();
-  if (tc && tc_rows_chain_supported(src, layers, n_layers, tc_passes(engine)) == DN_OK) {
-    return tc_rows_chain(src, layers, n_layers, V, tc_passes(engine), tc_ws, tc_ws_bytes, st);
-  }
+int run_chain(const DnRowsSrc& src, const DnLayer* layers, int n_layers, int64_t V, int tc, float* tmp0, float* tmp1,
+              void* tc_ws, int64_t tc_ws_bytes, cudaStream_t st) {
+  if (tc && tc_rows_chain_supported(src, layers, n_layers, tc) == DN_OK)
+    return tc_rows_chain(src, layers, n_layers, V, tc, tc_ws, tc_ws_bytes, st);
   // not fusable as a whole (e.g. a 256-wide layer inside a chain): layer by layer, each on the
   // tensor-core kernel when its shape allows, on the exact SIMT kernel otherwise
   DnRowsSrc cur = src;
@@ -89,10 +86,10 @@ int run_chain(const DnRowsSrc& src, DnLayer* layers, int n_layers, int64_t V, in
     }
     L.out = o; L.ld_out = ldo;
     int rc;
-    if (tc && tc_rows_chain_supported(cur, &L, 1, tc_passes(engine)) == DN_OK)
-      rc = tc_rows_chain(cur, &L, 1, V, tc_passes(engine), tc_ws, tc_ws_bytes, st);
+    if (tc && tc_rows_chain_supported(cur, &L, 1, tc) == DN_OK)
+      rc = tc_rows_chain(cur, &L, 1, V, tc, tc_ws, tc_ws_bytes, st);
     else {
-      if (use_tc(engine) && (rc = note_simt_fallback("a dense layer", L.K, L.N))) return rc;
+      if (tc && (rc = note_simt_fallback("a dense layer", L.K, L.N))) return rc;
       rc = simt_rows_gemm(cur, L, V, st);
     }
     if (rc) return rc;
@@ -101,23 +98,34 @@ int run_chain(const DnRowsSrc& src, DnLayer* layers, int n_layers, int64_t V, in
   return DN_OK;
 }
 
+// shapes the split-V tensor-core to_basis takes: up to 128 columns in one launch, wider (C_width = 256) in 128-column
+// slices
+bool to_basis_tc_fits(int K, int C) {
+  return tc_to_basis_supported(K, C) == DN_OK || (C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK);
+}
+
+// split-V to_basis partials on the tensor cores, for a shape to_basis_tc_fits accepts: wider than one accumulator set,
+// each 128-column slice is its own launch into the shared [P][K][C] partials.  With `batch`, grouped over a mesh batch:
+// every CTA reduces a row range inside one mesh (batch->tb_rows) into its own K x C partial.
+int to_basis_tc(const float* values, const float* basis, const float* massvec, int64_t V, int K, int C, float* partial,
+                int* P, int tc, cudaStream_t st, const dn_mesh_batch* batch = nullptr) {
+  const int32_t* cta_rows = batch ? batch->tb_rows : nullptr;
+  const int n_ctas = batch ? batch->n_tb_ctas : 0;
+  if (tc_to_basis_supported(K, C) == DN_OK)
+    return tc_to_basis_partial(values, basis, massvec, V, K, C, partial, P, tc, st, 0, 0, cta_rows, n_ctas);
+  for (int c0 = 0; c0 < C; c0 += 128) {
+    const int rc = tc_to_basis_partial(values + c0, basis, massvec, V, K, 128, partial + c0, P, tc, st, C, C, cta_rows,
+                                       n_ctas);
+    if (rc) return rc;
+  }
+  return DN_OK;
+}
+
 int to_basis_partials(const float* values, const float* basis, const float* massvec, int64_t V, int K, int C,
-                      float* partial, int64_t partial_floats, int* P, int engine, cudaStream_t st) {
-  if (use_tc(engine) && tc_supported_device() && tc_to_basis_supported(K, C) == DN_OK &&
-      (int64_t)148 * K * C <= partial_floats) {
-    return tc_to_basis_partial(values, basis, massvec, V, K, C, partial, P, tc_passes(engine), st);
-  }
-  // wider than one accumulator set (C_width = 256): 128-column slices, each its own launch into the shared partials
-  if (use_tc(engine) && tc_supported_device() && C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK &&
-      (int64_t)148 * K * C <= partial_floats) {
-    for (int c0 = 0; c0 < C; c0 += 128) {
-      const int rc = tc_to_basis_partial(values + c0, basis, massvec, V, K, 128, partial + c0, P, tc_passes(engine), st, C, C);
-      if (rc) return rc;
-    }
-    return DN_OK;
-  }
-  DN_TC_DEVICE_OR_FAIL(engine);
-  if (use_tc(engine)) { const int rc = note_simt_fallback("to_basis", K, C); if (rc) return rc; }
+                      float* partial, int64_t partial_floats, int* P, int tc, cudaStream_t st) {
+  if (tc && to_basis_tc_fits(K, C) && (int64_t)148 * K * C <= partial_floats)
+    return to_basis_tc(values, basis, massvec, V, K, C, partial, P, tc, st);
+  if (tc) { const int rc = note_simt_fallback("to_basis", K, C); if (rc) return rc; }
   // out[k][c] = sum_v basis[v][k] * (mass[v] * values[v][c])
   return simt_atb_partial_st(basis, K, K, values, C, C, massvec, V, partial, partial_floats, P, st);
 }
@@ -126,62 +134,39 @@ int to_basis_partials(const float* values, const float* basis, const float* mass
 // Tensor cores (the split-V to_basis kernel, reference geometry.py:572-583 has the same contraction) when both
 // operands are contiguous and at most 128 wide; the exact SIMT kernel otherwise.
 int atb(const float* A, int64_t lda, int I, const float* B, int64_t ldb, int J, int64_t V, float* out, int64_t ld_out,
-        int accumulate, float* part, int64_t part_floats, int engine, cudaStream_t st) {
-  if (use_tc(engine) && tc_supported_device() && lda == I && ldb == J && tc_to_basis_supported(I, J) == DN_OK &&
-      (int64_t)148 * I * J <= part_floats) {
+        int accumulate, float* part, int64_t part_floats, int tc, cudaStream_t st) {
+  if (tc && lda == I && ldb == J && tc_to_basis_supported(I, J) == DN_OK && (int64_t)148 * I * J <= part_floats) {
     int P = 0;
-    int rc = tc_to_basis_partial(B, A, nullptr, V, I, J, part, &P, tc_passes(engine), st);
+    int rc = tc_to_basis_partial(B, A, nullptr, V, I, J, part, &P, tc, st);
     if (rc == DN_OK) return launch_reduce_partials_ld(part, P, I, J, out, ld_out, accumulate, st);
     if (rc != DN_ERR_UNSUPPORTED) return rc;
   }
-  DN_TC_DEVICE_OR_FAIL(engine);
-  if (use_tc(engine)) { const int rc = note_simt_fallback("a weight gradient", I, J); if (rc) return rc; }
+  if (tc) { const int rc = note_simt_fallback("a weight gradient", I, J); if (rc) return rc; }
   return simt_atb(A, lda, I, B, ldb, J, nullptr, V, out, ld_out, accumulate, part, part_floats, st);
 }
 
-// one dense layer on the tensor-core chain kernel when it takes the shape, else the exact SIMT kernel
-int one_layer(const DnRowsSrc& src, DnLayer& L, int64_t V, int engine, void* tc_ws, int64_t tc_ws_bytes, cudaStream_t st) {
-  if (use_tc(engine) && tc_supported_device() && tc_rows_chain_supported(src, &L, 1, tc_passes(engine)) == DN_OK)
-    return tc_rows_chain(src, &L, 1, V, tc_passes(engine), tc_ws, tc_ws_bytes, st);
-  DN_TC_DEVICE_OR_FAIL(engine);
-  if (use_tc(engine)) { const int rc = note_simt_fallback("a dense layer", L.K, L.N); if (rc) return rc; }
-  return simt_rows_gemm(src, L, V, st);
-}
-
-// grouped split-V to_basis over a mesh batch: every CTA reduces a row range inside one mesh (batch->tb_rows) into its
-// own K x C partial; C_width = 256 runs as two 128-column launches into the same partials
-int grouped_to_basis(const float* values, const float* basis, const float* massvec, int64_t V, int K, int C,
-                     float* partial, const dn_mesh_batch* batch, int engine, cudaStream_t st) {
-  int P = 0;
-  if (tc_to_basis_supported(K, C) == DN_OK)
-    return tc_to_basis_partial(values, basis, massvec, V, K, C, partial, &P, tc_passes(engine), st, 0, 0, batch->tb_rows,
-                               batch->n_tb_ctas);
-  if (!(C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK)) return DN_ERR_UNSUPPORTED;
-  for (int c0 = 0; c0 < C; c0 += 128) {
-    const int rc = tc_to_basis_partial(values + c0, basis, massvec, V, K, 128, partial + c0, &P, tc_passes(engine), st, C,
-                                       C, batch->tb_rows, batch->n_tb_ctas);
-    if (rc) return rc;
-  }
+// A mesh batch (dn_mesh_batch_plan) laid out as one vertex range, and the grouped to_basis of `values` over it, checked
+// before anything is enqueued: every descriptor field set, whole 128-row tiles, 16-byte aligned `values` / `evecs`,
+// K and C inside the split-V kernel.
+int check_batch(const dn_mesh_batch* batch, const float* values, const float* evecs, int64_t V, int K, int C) {
+  if (!batch || batch->n_meshes < 1 || batch->n_tb_ctas < 1 || !batch->tile_mesh || !batch->tb_rows ||
+      !batch->mesh_cta_begin)
+    return DN_ERR_INVALID_ARGUMENT;
+  if ((V % 128) || V >= (1ll << 31) - 256 || (C % 4) || (reinterpret_cast<uintptr_t>(values) & 15) ||
+      (reinterpret_cast<uintptr_t>(evecs) & 15) || !to_basis_tc_fits(K, C))
+    return DN_ERR_UNSUPPORTED;
   return DN_OK;
 }
 
 // Support checks of the grouped spectral stage (learned-time diffusion over a mesh batch), all made before anything is
-// enqueued: the grouped to_basis, and a from_basis chain `L` that picks its weights per tile.  Chooses L's pack format.
+// enqueued: the batch, and a from_basis chain `L` that picks its weights per tile.  Chooses L's pack format.
 int grouped_spectral_check(const float* values, const float* evecs, const dn_mesh_batch* batch, int64_t V, int K, int C,
-                           int engine, DnLayer* L) {
-  if (!batch || batch->n_meshes < 1 || batch->n_tb_ctas < 1 || !batch->tile_mesh || !batch->tb_rows ||
-      !batch->mesh_cta_begin)
-    return DN_ERR_INVALID_ARGUMENT;
-  if (!use_tc(engine)) return DN_ERR_UNSUPPORTED;
-  if (!tc_supported_device()) return DN_ERR_NOT_SM100;
-  if ((V % 128) || V >= (1ll << 31) - 256 || (C % 4) || (reinterpret_cast<uintptr_t>(values) & 15) ||
-      (reinterpret_cast<uintptr_t>(evecs) & 15))
-    return DN_ERR_UNSUPPORTED;
-  if (tc_to_basis_supported(K, C) != DN_OK && !(C > 128 && C % 128 == 0 && tc_to_basis_supported(K, 128) == DN_OK))
-    return DN_ERR_UNSUPPORTED;
+                           int tc, DnLayer* L) {
+  const int rc = check_batch(batch, values, evecs, V, K, C);
+  if (rc) return rc;
   const DnRowsSrc src = one_src(evecs, K, K);
-  if (tc_grouped_chain_supported(src, L, 1, tc_passes(engine)) != DN_OK) return DN_ERR_UNSUPPORTED;
-  tc_choose_pack_fmt(src, L, 1, tc_passes(engine));
+  if (!tc || tc_grouped_chain_supported(src, L, 1, tc) != DN_OK) return DN_ERR_UNSUPPORTED;
+  tc_choose_pack_fmt(src, L, 1, tc);
   return DN_OK;
 }
 
@@ -341,24 +326,27 @@ int dn_compute_hks(const float* evals, const float* evecs, const float* scales, 
 int dn_to_basis(const float* values, const float* basis, const float* massvec, int64_t V, int K, int C, float* out,
                 void* workspace, int64_t ws_bytes, int engine, dn_stream_t stream) {
   if (!values || !basis || !out || V < 0 || K <= 0 || C <= 0) return DN_ERR_INVALID_ARGUMENT;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   const int64_t pf = ws.left_floats() < kPartialFloats ? ws.left_floats() : kPartialFloats;
   float* partial = ws.take(pf);
   if (!partial) return DN_ERR_WORKSPACE;
   int P = 0;
-  int rc = to_basis_partials(values, basis, massvec, V, K, C, partial, pf, &P, engine, st);
-  if (rc) return rc;
+  if ((rc = to_basis_partials(values, basis, massvec, V, K, C, partial, pf, &P, tc, st))) return rc;
   return launch_reduce_partials(partial, P, (int64_t)K * C, out, st);
 }
 
 int dn_from_basis(const float* values, const float* basis, const float* row_scale, int64_t V, int K, int C,
                   float* out, void* workspace, int64_t ws_bytes, int engine, dn_stream_t stream) {
   if (!values || !basis || !out || V < 0 || K <= 0 || C <= 0) return DN_ERR_INVALID_ARGUMENT;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   DnRowsSrc src = one_src(basis, K, K);
   DnLayer L = make_layer(values, C, /*w_trans=*/1, nullptr, 0, K, C, out, C);
   L.row_scale = row_scale;
-  return run_chain(src, &L, 1, V, engine, nullptr, nullptr, workspace, ws_bytes, (cudaStream_t)stream);
+  return run_chain(src, &L, 1, V, tc, nullptr, nullptr, workspace, ws_bytes, (cudaStream_t)stream);
 }
 
 int dn_learned_time_diffusion_fwd(const float* x, const float* mass, const float* evals, const float* evecs,
@@ -366,6 +354,8 @@ int dn_learned_time_diffusion_fwd(const float* x, const float* mass, const float
                                   void* workspace, int64_t ws_bytes, int engine, dn_stream_t stream) {
   if (!x || !mass || !evals || !evecs || !time || !x_diffuse || V < 0 || K <= 0 || C <= 0)
     return DN_ERR_INVALID_ARGUMENT;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   float* S = ws.take((int64_t)K * C);
@@ -373,13 +363,12 @@ int dn_learned_time_diffusion_fwd(const float* x, const float* mass, const float
   float* partial = ws.take(pf);
   if (!S || !partial) return DN_ERR_WORKSPACE;
   int P = 0;
-  int rc = to_basis_partials(x, evecs, mass, V, K, C, partial, pf, &P, engine, st);
-  if (rc) return rc;
+  if ((rc = to_basis_partials(x, evecs, mass, V, K, C, partial, pf, &P, tc, st))) return rc;
   rc = launch_spectral_scale(partial, P, evals, time, K, C, x_spec_out, S, /*clamp_writeback=*/1, st);
   if (rc) return rc;
   DnRowsSrc src = one_src(evecs, K, K);
   DnLayer L = make_layer(S, C, 1, nullptr, 0, K, C, x_diffuse, C);
-  return run_chain(src, &L, 1, V, engine, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st);
+  return run_chain(src, &L, 1, V, tc, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st);
 }
 
 int dn_learned_time_diffusion_bwd(const float* grad_out, const float* mass, const float* evals, const float* evecs,
@@ -388,6 +377,8 @@ int dn_learned_time_diffusion_bwd(const float* grad_out, const float* mass, cons
                                   dn_stream_t stream) {
   if (!grad_out || !mass || !evals || !evecs || !time || !x_spec || !grad_x || !grad_time)
     return DN_ERR_INVALID_ARGUMENT;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   float* dS = ws.take((int64_t)K * C);
@@ -395,8 +386,7 @@ int dn_learned_time_diffusion_bwd(const float* grad_out, const float* mass, cons
   float* partial = ws.take(pf);
   if (!dS || !partial) return DN_ERR_WORKSPACE;
   int P = 0;
-  int rc = to_basis_partials(grad_out, evecs, nullptr, V, K, C, partial, pf, &P, engine, st);
-  if (rc) return rc;
+  if ((rc = to_basis_partials(grad_out, evecs, nullptr, V, K, C, partial, pf, &P, tc, st))) return rc;
   if (P > 4) {
     // spectral_bwd walks the partials serially per channel: with the 148 split-V partials of the tensor-core kernel that
     // took 4.5 ms (V = 7k); sum them first (coalesced, parallel) and hand it one
@@ -411,7 +401,7 @@ int dn_learned_time_diffusion_bwd(const float* grad_out, const float* mass, cons
   DnRowsSrc src = one_src(evecs, K, K);
   DnLayer L = make_layer(dS, C, 1, nullptr, 0, K, C, grad_x, C);
   L.row_scale = mass;
-  return run_chain(src, &L, 1, V, engine, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st);
+  return run_chain(src, &L, 1, V, tc, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st);
 }
 
 int dn_learned_time_diffusion_fwd_batched(const float* x, const float* mass, const float* evals, const float* evecs,
@@ -421,8 +411,8 @@ int dn_learned_time_diffusion_fwd_batched(const float* x, const float* mass, con
   if (!x || !mass || !evals || !evecs || !time || !x_diffuse || V < 0 || K <= 0 || C <= 0)
     return DN_ERR_INVALID_ARGUMENT;
   DnLayer L = make_layer(nullptr, C, /*w_trans=*/1, nullptr, 0, K, C, x_diffuse, C);
-  int rc = grouped_spectral_check(x, evecs, batch, V, K, C, engine, &L);
-  if (rc) return rc;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc || (rc = grouped_spectral_check(x, evecs, batch, V, K, C, tc, &L))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   const int64_t pb = tc_chain_ws_bytes(&L, 1) * batch->n_meshes;
@@ -430,11 +420,12 @@ int dn_learned_time_diffusion_fwd_batched(const float* x, const float* mass, con
   float* partial = ws.take((int64_t)batch->n_tb_ctas * K * C);
   if (!pk || !partial) return DN_ERR_WORKSPACE;
   // (nothing has been enqueued up to here)
-  if ((rc = grouped_to_basis(x, evecs, mass, V, K, C, partial, batch, engine, st))) return rc;
+  int P = 0;
+  if ((rc = to_basis_tc(x, evecs, mass, V, K, C, partial, &P, tc, st, batch))) return rc;
   if ((rc = tc_pack_spectral_batched(&L, batch->n_meshes, pk, pb, partial, batch->mesh_cta_begin, evals, time,
                                      /*clamp_writeback=*/1, batch->tile_mesh, st, x_spec_out)))
     return rc;
-  return tc_rows_chain(one_src(evecs, K, K), &L, 1, V, tc_passes(engine), ws.base + ws.off, ws.size - ws.off, st);
+  return tc_rows_chain(one_src(evecs, K, K), &L, 1, V, tc, ws.base + ws.off, ws.size - ws.off, st);
 }
 
 int dn_learned_time_diffusion_bwd_batched(const float* grad_out, const float* mass, const float* evals,
@@ -447,8 +438,8 @@ int dn_learned_time_diffusion_bwd_batched(const float* grad_out, const float* ma
   // grad_x = mass * (Phi_b dS_b) per tile: the from_basis chain with per-mesh weights and a row_scale epilogue
   DnLayer L = make_layer(nullptr, C, /*w_trans=*/1, nullptr, 0, K, C, grad_x, C);
   L.row_scale = mass;
-  int rc = grouped_spectral_check(grad_out, evecs, batch, V, K, C, engine, &L);
-  if (rc) return rc;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc || (rc = grouped_spectral_check(grad_out, evecs, batch, V, K, C, tc, &L))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   const int64_t pb = tc_chain_ws_bytes(&L, 1) * batch->n_meshes;
@@ -457,11 +448,12 @@ int dn_learned_time_diffusion_bwd_batched(const float* grad_out, const float* ma
   float* partial = ws.take((int64_t)batch->n_tb_ctas * K * C);
   if (!pk || !dt || !partial) return DN_ERR_WORKSPACE;
   // (nothing has been enqueued up to here)
-  if ((rc = grouped_to_basis(grad_out, evecs, nullptr, V, K, C, partial, batch, engine, st))) return rc;
+  int P = 0;
+  if ((rc = to_basis_tc(grad_out, evecs, nullptr, V, K, C, partial, &P, tc, st, batch))) return rc;
   if ((rc = tc_spectral_bwd_batched(&L, batch->n_meshes, pk, pb, partial, batch->mesh_cta_begin, evals, time, x_spec, dt,
                                     grad_time, batch->tile_mesh, st)))
     return rc;
-  return tc_rows_chain(one_src(evecs, K, K), &L, 1, V, tc_passes(engine), ws.base + ws.off, ws.size - ws.off, st);
+  return tc_rows_chain(one_src(evecs, K, K), &L, 1, V, tc, ws.base + ws.off, ws.size - ws.off, st);
 }
 
 int dn_grad_spmm(const dn_csr* grad, const float* x, int64_t V, int C, float* out, dn_stream_t stream) {
@@ -511,6 +503,8 @@ int dn_gradient_features_fwd(const dn_csr* grad, const float* x_diffuse, const f
       C <= 0)
     return DN_ERR_INVALID_ARGUMENT;
   if (C % 4) return DN_ERR_UNSUPPORTED;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   const int npq = with_gradient_rotations ? 2 * C : C;
@@ -519,8 +513,7 @@ int dn_gradient_features_fwd(const dn_csr* grad, const float* x_diffuse, const f
   DnRowsSrc src = one_src(x_diffuse, C, C);
   DnLayer L = make_layer(A_re, C, 0, nullptr, 0, C, npq, pq, npq);   // [P|Q] = xd [A_re;A_im]^T
   if (with_gradient_rotations) { L.W2 = A_im; L.n_split = C; }
-  int rc = run_chain(src, &L, 1, V, engine, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st);
-  if (rc) return rc;
+  if ((rc = run_chain(src, &L, 1, V, tc, nullptr, nullptr, ws.base + ws.off, ws.size - ws.off, st))) return rc;
   return launch_spmm_features(grad, x_diffuse, pq, with_gradient_rotations, V, C, features, st);
 }
 
@@ -533,6 +526,8 @@ int dn_gradient_features_bwd(const dn_csr* grad, const dn_csr* grad_t, const flo
       (with_gradient_rotations && (!A_im || !grad_A_im)))
     return DN_ERR_INVALID_ARGUMENT;
   if (C % 4) return DN_ERR_UNSUPPORTED;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   const int rot = with_gradient_rotations;
@@ -544,7 +539,6 @@ int dn_gradient_features_bwd(const dn_csr* grad, const dn_csr* grad_t, const flo
   if (!U || !dxd || !dP || (rot && !dQ) || !part) return DN_ERR_WORKSPACE;
   void* tcws = ws.base + ws.off;
   const int64_t tcws_bytes = ws.size - ws.off;
-  int rc;
   if ((rc = launch_features_bwd_local(grad, x_diffuse, pq, features, grad_features, rot, V, C, U, st))) return rc;
   if ((rc = launch_features_bwd_transpose(grad_t, U, rot, V, C, dxd, dP, dQ, C, st))) return rc;
   // grad_x = dxd + dP A_re (+ dQ A_im): one layer over the sources (dP | dQ) with [A_re ; A_im] stacked along K
@@ -556,9 +550,10 @@ int dn_gradient_features_bwd(const dn_csr* grad, const dn_csr* grad_t, const flo
     DnLayer L = make_layer(A_re, C, /*w_trans=*/1, nullptr, 0, rot ? 2 * C : C, C, grad_x, C);
     if (rot) { L.W2 = A_im; L.n_split = C; }
     L.residual = dxd; L.ld_res = C;
-    if (use_tc(engine) && tc_supported_device() && tc_rows_chain_supported(s, &L, 1, tc_passes(engine)) == DN_OK) {
-      if ((rc = tc_rows_chain(s, &L, 1, V, tc_passes(engine), tcws, tcws_bytes, st))) return rc;
+    if (tc && tc_rows_chain_supported(s, &L, 1, tc) == DN_OK) {
+      if ((rc = tc_rows_chain(s, &L, 1, V, tc, tcws, tcws_bytes, st))) return rc;
     } else {                                       // exact SIMT route: one source at a time
+      if (tc && (rc = note_simt_fallback("a dense layer", L.K, L.N))) return rc;
       DnRowsSrc s0 = one_src(dP, C, C);
       DnLayer L0 = make_layer(A_re, C, 1, nullptr, 0, C, C, grad_x, C);
       L0.residual = dxd; L0.ld_res = C;
@@ -572,9 +567,9 @@ int dn_gradient_features_bwd(const dn_csr* grad, const dn_csr* grad_t, const flo
     }
   }
   // grad_A_re[n][k] += sum_v dP[v][n] xd[v][k]   (and grad_A_im from dQ)
-  if ((rc = atb(dP, C, C, x_diffuse, C, C, V, grad_A_re, C, 1, part, kPartialFloats / 4, engine, st))) return rc;
+  if ((rc = atb(dP, C, C, x_diffuse, C, C, V, grad_A_re, C, 1, part, kPartialFloats / 4, tc, st))) return rc;
   if (rot)
-    if ((rc = atb(dQ, C, C, x_diffuse, C, C, V, grad_A_im, C, 1, part, kPartialFloats / 4, engine, st))) return rc;
+    if ((rc = atb(dQ, C, C, x_diffuse, C, C, V, grad_A_im, C, 1, part, kPartialFloats / 4, tc, st))) return rc;
   return DN_OK;
 }
 
@@ -586,6 +581,8 @@ int dn_mini_mlp_fwd(const float* const* src_host, const int* src_width_host, int
   if (!src_host || !src_width_host || nsrc < 1 || nsrc > DN_MAX_SRC || !weight_host || !dims_host || n_layers < 1 ||
       n_layers > DN_MAX_LAYERS || !out || V < 0)
     return DN_ERR_INVALID_ARGUMENT;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   DnRowsSrc src;
   memset(&src, 0, sizeof(src));
   int k0 = 0;
@@ -610,14 +607,13 @@ int dn_mini_mlp_fwd(const float* const* src_host, const int* src_width_host, int
   }
   Bump ws(workspace, ws_bytes);
   float *t0 = nullptr, *t1 = nullptr;
-  const bool fused = use_tc(engine) && tc_supported_device() && tc_rows_chain_supported(src, layers, n_layers, tc_passes(engine)) == DN_OK;
+  const bool fused = tc && tc_rows_chain_supported(src, layers, n_layers, tc) == DN_OK;
   if (!fused && n_layers > 1) {
     t0 = ws.take(V * maxn);
     t1 = ws.take(V * maxn);
     if (!t0 || !t1) return DN_ERR_WORKSPACE;
   }
-  return run_chain(src, layers, n_layers, V, engine, t0, t1, ws.base + ws.off, ws.size - ws.off,
-                   (cudaStream_t)stream);
+  return run_chain(src, layers, n_layers, V, tc, t0, t1, ws.base + ws.off, ws.size - ws.off, (cudaStream_t)stream);
 }
 
 int dn_mini_mlp_bwd(const float* grad_out, const float* const* src_host, const int* src_width_host, int nsrc,
@@ -629,6 +625,8 @@ int dn_mini_mlp_bwd(const float* grad_out, const float* const* src_host, const i
       n_layers < 1 || n_layers > DN_MAX_LAYERS || (n_layers > 1 && !hidden_host) || !grad_src_host ||
       !grad_weight_host)
     return DN_ERR_INVALID_ARGUMENT;
+  int tc, rc = resolve_engine(engine, &tc);
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   int maxn = 0;
   for (int l = 0; l <= n_layers; ++l) maxn = dims_host[l] > maxn ? dims_host[l] : maxn;
@@ -640,19 +638,18 @@ int dn_mini_mlp_bwd(const float* grad_out, const float* const* src_host, const i
   void* tcws = ws.base + ws.off;
   const int64_t tcws_bytes = ws.size - ws.off;
   const float* dz = grad_out;   // gradient w.r.t. the pre-activation of layer l
-  int rc;
   for (int l = n_layers - 1; l >= 0; --l) {
     const int nout = dims_host[l + 1], nin = dims_host[l];
     // weight / bias gradients:  grad_W[n][k] += sum_v dz[v][n] * h_{l-1}[v][k]
     if (l > 0) {
       if ((rc = atb(dz, nout, nout, hidden_host[l - 1], nin, nin, V, grad_weight_host[l], nin, 1, part,
-                    kPartialFloats / 2, engine, st)))
+                    kPartialFloats / 2, tc, st)))
         return rc;
     } else {
       int off = 0;
       for (int s = 0; s < nsrc; ++s) {
         if ((rc = atb(dz, nout, nout, src_host[s], src_width_host[s], src_width_host[s], V, grad_weight_host[0] + off,
-                      nin, 1, part, kPartialFloats / 2, engine, st)))
+                      nin, 1, part, kPartialFloats / 2, tc, st)))
           return rc;
         off += src_width_host[s];
       }
@@ -666,7 +663,7 @@ int dn_mini_mlp_bwd(const float* grad_out, const float* const* src_host, const i
       DnLayer L = make_layer(weight_host[l], nin, /*w_trans=*/1, nullptr, 0, nout, nin, o, nin);
       L.relu_mask_src = hidden_host[l - 1];
       if (drop_mask_host && drop_mask_host[l - 1]) L.emul = drop_mask_host[l - 1];
-      if ((rc = one_layer(s, L, V, engine, tcws, tcws_bytes, st))) return rc;
+      if ((rc = run_chain(s, &L, 1, V, tc, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
       dz = o;
     } else {
       int off = 0;
@@ -674,7 +671,7 @@ int dn_mini_mlp_bwd(const float* grad_out, const float* const* src_host, const i
         if (grad_src_host[q]) {
           DnLayer L = make_layer(weight_host[0] + off, nin, 1, nullptr, 0, nout, src_width_host[q], grad_src_host[q],
                                  src_width_host[q]);
-          if ((rc = one_layer(s, L, V, engine, tcws, tcws_bytes, st))) return rc;
+          if ((rc = run_chain(s, &L, 1, V, tc, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
         }
         off += src_width_host[q];
       }
@@ -698,6 +695,8 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
   if (p->n_mlp_layers < 1 || p->n_mlp_layers > DN_MAX_LAYERS || !p->mlp_weight_host || !p->mlp_dims_host)
     return DN_ERR_INVALID_ARGUMENT;
   if (p->with_gradient_features && (C % 4)) return DN_ERR_UNSUPPORTED;
+  int tc, rc = resolve_engine(engine, &tc), P = 0;
+  if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   Bump ws(workspace, ws_bytes);
   const int rot = p->with_gradient_rotations;
@@ -709,7 +708,6 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
   const int64_t pf = kPartialFloats;
   float* partial = ws.take(pf);
   if (!S || !xd || !partial || (p->with_gradient_features && (!pq || !feat))) return DN_ERR_WORKSPACE;
-  int rc, P = 0;
 
   // every dense layer of the block: [0] from_basis, [1] (a5, commuted) [P|Q] = x_diffuse [A_re;A_im]^T,
   // [2..] cat -> MiniMLP -> + x_in  [layers.py:229-239]
@@ -720,21 +718,19 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
   // Tensor-core gradient features (C_width = 128, learned rotations, fp32-grade / TF32 engines): gather only x_diffuse
   // (gxy = [gradX x | gradY x], a third of the commuted route's gather traffic), then the complex-linear map as tcgen05
   // GEMMs whose epilogue forms tanh(gX * Bre + gY * Bim) (layers.py:117-130) -- two launches of 64 channels each, so
-  // that the [Bre | Bim] accumulators (128 columns) ping-pong in TMEM.  DN_GF_TC=0 restores the commuted route
+  // that the [Bre | Bim] accumulators (128 columns) ping-pong in TMEM.  Every other block takes the commuted route
   // ([P|Q] = x_diffuse [A_re; A_im]^T in front of a gather of x, P and Q).
-  static int gf_env = -1;
-  if (gf_env < 0) { const char* e = getenv("DN_GF_TC"); gf_env = (!e || atoi(e) != 0) ? 1 : 0; }
   bool gf_tc = false;
   DnRowsSrc src_gxy = one_src(pq, 2 * C, 2 * C);
-  if (p->with_gradient_features && rot && C == 128 && gf_env && use_tc(engine) && engine != DN_ENGINE_BF16 &&
-      tc_supported_device() && !(grad->patches && grad->patches->n_patches > 0)) {
+  if (p->with_gradient_features && rot && C == 128 && tc && tc != DN_PASSES_BF16 &&
+      !(grad->patches && grad->patches->n_patches > 0)) {
     for (int h = 0; h < 2; ++h) {
       L[1 + h] = make_layer(p->A_re, C, 0, nullptr, 0, 2 * C, C, feat + h * 64, C);
       L[1 + h].W2 = p->A_im; L[1 + h].rot_C = C; L[1 + h].rot_ch0 = h * 64;
       L[1 + h].dots_src = pq + h * 64; L[1 + h].ld_dots = 2 * C; L[1 + h].dots_gy_col = C;
     }
-    gf_tc = tc_rows_chain_supported(src_gxy, &L[1], 1, tc_passes(engine)) == DN_OK &&
-            tc_rows_chain_supported(src_gxy, &L[2], 1, tc_passes(engine)) == DN_OK;
+    gf_tc = tc_rows_chain_supported(src_gxy, &L[1], 1, tc) == DN_OK &&
+            tc_rows_chain_supported(src_gxy, &L[2], 1, tc) == DN_OK;
     if (gf_tc) nfront = 3;
   }
   if (p->with_gradient_features && !gf_tc) {
@@ -778,31 +774,29 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
   for (int q = 0; q < nsrc; ++q) { src_mlp.ptr[q] = srcs[q]; src_mlp.width[q] = C; src_mlp.ld[q] = C; }
   src_mlp.nsrc = nsrc;
   // one launch packs (hi/lo split + UMMA layout) every weight the tensor-core kernels will stream
-  const bool tc = use_tc(engine) && tc_supported_device();
-  const int passes = tc_passes(engine);
-  const bool front_fused = tc && nfront == 2 && tc_rows_chain_supported(src_fb, &L[0], 2, passes) == DN_OK;
+  const bool front_fused = tc && nfront == 2 && tc_rows_chain_supported(src_fb, &L[0], 2, tc) == DN_OK;
   bool tc_front = front_fused;
   const DnRowsSrc& src_l12 = gf_tc ? src_gxy : src_pq;      // input of L[1], L[2]: raw gradients | x_diffuse
   if (tc && !front_fused) {
-    tc_front = tc_rows_chain_supported(src_fb, &L[0], 1, passes) == DN_OK;
-    for (int l = 1; l < nfront; ++l) tc_front = tc_front && tc_rows_chain_supported(src_l12, &L[l], 1, passes) == DN_OK;
+    tc_front = tc_rows_chain_supported(src_fb, &L[0], 1, tc) == DN_OK;
+    for (int l = 1; l < nfront; ++l) tc_front = tc_front && tc_rows_chain_supported(src_l12, &L[l], 1, tc) == DN_OK;
   }
   if (gf_tc && !tc_front) return DN_ERR_UNSUPPORTED;         // (from_basis outside the envelope: cannot happen at C = 128)
-  const bool tc_mlp = tc && tc_rows_chain_supported(src_mlp, &L[nfront], nm, passes) == DN_OK;
+  const bool tc_mlp = tc && tc_rows_chain_supported(src_mlp, &L[nfront], nm, tc) == DN_OK;
   if (head && !tc_mlp) return DN_ERR_UNSUPPORTED;
   // the spectral multiplier S = exp(-lambda t) * (reduced partial sums) is layer 0's weight: when the tensor-core path
   // takes the front chain it is formed inside the pack launch (no separate scale kernel, S never round-trips HBM)
-  if (batch && !tc_front) return DN_ERR_UNSUPPORTED;
+  if (batch) {
+    if ((rc = check_batch(batch, x_in, evecs, V, K, C))) return rc;
+    if (!tc_front || (int64_t)batch->n_tb_ctas * K * C > pf) return DN_ERR_UNSUPPORTED;
+  }
   // (nothing has been launched up to here: an unsupported head / batch returns before any work is enqueued)
   mark(0);
-  // (a1) spectral diffusion: to_basis -> exp(-lambda t) -> from_basis   [layers.py:56-67]
+  // (a1) spectral diffusion: to_basis -> exp(-lambda t) -> from_basis   [layers.py:56-67]; over a batch the grouped
+  // split-V to_basis, every CTA reducing a row range inside one mesh
   if (batch) {
-    // grouped split-V: every CTA reduces a row range inside one mesh
-    if (!use_tc(engine) || !tc_supported_device() || (V % 128) || batch->n_meshes < 1 || !batch->tile_mesh ||
-        !batch->tb_rows || !batch->mesh_cta_begin || batch->n_tb_ctas < 1 || (int64_t)batch->n_tb_ctas * K * C > pf)
-      return DN_ERR_UNSUPPORTED;
-    if ((rc = grouped_to_basis(x_in, evecs, mass, V, K, C, partial, batch, engine, st))) return rc;
-  } else if ((rc = to_basis_partials(x_in, evecs, mass, V, K, C, partial, pf, &P, engine, st))) {
+    if ((rc = to_basis_tc(x_in, evecs, mass, V, K, C, partial, &P, tc, st, batch))) return rc;
+  } else if ((rc = to_basis_partials(x_in, evecs, mass, V, K, C, partial, pf, &P, tc, st))) {
     return rc;
   }
   mark(1);
@@ -810,13 +804,13 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
     if ((rc = launch_spectral_scale(partial, P, evals, p->diffusion_time, K, C, nullptr, S, 1, st))) return rc;
   mark(2);
   if (tc_front) {
-    if (front_fused) tc_choose_pack_fmt(src_fb, &L[0], 2, passes);
+    if (front_fused) tc_choose_pack_fmt(src_fb, &L[0], 2, tc);
     else {
-      tc_choose_pack_fmt(src_fb, &L[0], 1, passes);
-      for (int l = 1; l < nfront; ++l) tc_choose_pack_fmt(src_l12, &L[l], 1, passes);
+      tc_choose_pack_fmt(src_fb, &L[0], 1, tc);
+      for (int l = 1; l < nfront; ++l) tc_choose_pack_fmt(src_l12, &L[l], 1, tc);
     }
   }
-  if (tc_mlp) tc_choose_pack_fmt(src_mlp, &L[nfront], nm, passes);
+  if (tc_mlp) tc_choose_pack_fmt(src_mlp, &L[nfront], nm, tc);
   if (batch) {
     // one packed spectral multiplier per mesh (layer 0 of the front chain picks its matrix per tile), then every other
     // weight of the block in one more launch
@@ -855,12 +849,12 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
   const int64_t tcws_bytes = ws.size - ws.off;
   // from_basis and [P|Q]: one fused two-layer chain when it fits, else one launch per layer
   if (front_fused) {
-    if ((rc = run_chain(src_fb, &L[0], 2, V, engine, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
+    if ((rc = run_chain(src_fb, &L[0], 2, V, tc, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
   } else {
-    if ((rc = run_chain(src_fb, &L[0], 1, V, engine, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
+    if ((rc = run_chain(src_fb, &L[0], 1, V, tc, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
     if (!gf_tc)
       for (int l = 1; l < nfront; ++l)
-        if ((rc = run_chain(src_pq, &L[l], 1, V, engine, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
+        if ((rc = run_chain(src_pq, &L[l], 1, V, tc, nullptr, nullptr, tcws, tcws_bytes, st))) return rc;
   }
   mark(4);
   // (a4+a5) sparse tangent gradient + complex inner product + tanh   [layers.py:216-226,128-130]
@@ -871,12 +865,12 @@ static int block_fwd_impl(const float* x_in, const float* mass, const float* eva
       if (g_gf_ev) { cudaEventRecord(g_gf_ev, st); g_gf_recorded = true; }
     }
     for (int l = 1; l < nfront; ++l)
-      if ((rc = tc_rows_chain(src_gxy, &L[l], 1, V, passes, tcws, tcws_bytes, st))) return rc;
+      if ((rc = tc_rows_chain(src_gxy, &L[l], 1, V, tc, tcws, tcws_bytes, st))) return rc;
   } else if (p->with_gradient_features) {
     if ((rc = launch_spmm_features(grad, xd, pq, rot, V, C, feat, st))) return rc;
   }
   mark(5);
-  rc = run_chain(src_mlp, &L[nfront], nm, V, engine, t0, t1, tcws, tcws_bytes, st);
+  rc = run_chain(src_mlp, &L[nfront], nm, V, tc, t0, t1, tcws, tcws_bytes, st);
   mark(6);
   return rc;
 }

@@ -4,12 +4,13 @@
 //     cat(x_in, x_diffuse, features) -> MiniMLP -> + x_in              reference layers.py:133-164, 229-239
 //
 // One persistent CTA per SM, 16 warps, every role fed by an mbarrier ring:
-//   warp 0      weight producer: one bulk copy (cp.async.bulk) per 32-wide K-stage of pre-split (hi | lo) weights
+//   warp 0      weight producer: one bulk copy (cp.async.bulk) per 32-wide K-stage of pre-split weights
+//               ([tf32 hi | bf16 (hi ; lo)], pack format 1)
 //   warp 1      row-box producer: layer-0 operands as 128-row x 32-column fp32 boxes through TMA tensor maps
 //               (SWIZZLE_128B), four slots
-//   warp 2      MMA issuer: tcgen05.mma.kind::tf32, A operand from TENSOR MEMORY, B from shared memory, twelve MMAs
-//               (4 k-steps x {lo*hi, hi*lo, hi*hi}) per hand-off and ONE tcgen05.commit that releases the TMEM operand
-//               stage and the weight stage together
+//   warp 2      MMA issuer, A operand from TENSOR MEMORY, B from shared memory: per 32-wide stage four
+//               tcgen05.mma.kind::tf32 (hi*hi) and, fp32-grade, four kind::f16 bf16 MMAs for the correction terms, then
+//               ONE tcgen05.commit that releases the TMEM operand stage and the weight stage together
 //   warp 3      allocates / frees TMEM
 //   warps 4-11  two operand warpgroups.  Stage c of every layer belongs to warpgroup c & 1 (so each ring slot has a
 //               single in-order producer -- the mbarrier parity protocol needs that): layer-0 stages are read back
@@ -35,7 +36,6 @@
 #include "dn_internal.h"
 #include "dn_tc_ptx.cuh"
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -46,16 +46,19 @@ constexpr int C3_THREADS = 512;
 constexpr int C3_KS = 32;                       // k-columns per pipeline stage
 constexpr int C3_TILE = 128;                    // rows per tile == UMMA M
 constexpr int C3_RAW = C3_TILE * C3_KS * 4;     // 16 KiB row box
-// row-box slots + output staging buffers share 6 x 16 KiB: 4 + 2 (default: layer 0 is long, the output is short) or
-// 2 + 4 (from_basis -> [P|Q]: four layer-0 stages per tile, 192 KiB of output per tile)
+// row-box slots + output staging buffers share 6 x 16 KiB: 4 + 2.  (2 + 4 was measured on the output-heavy
+// from_basis -> [P|Q] chain -- four layer-0 stages, 192 KiB of output per tile -- and was SLOWER, 124 vs 108 us: the
+// extra staging traffic competes with the tensor core for shared-memory bandwidth.)
 constexpr int C3_IO_BUFS = 6;
+constexpr int C3_RAW_SHIFT = 2;                 // row-box slots = 1 << C3_RAW_SHIFT
+constexpr int C3_RAW_SLOTS = 1 << C3_RAW_SHIFT;
 constexpr int C3_WBYTES = 131072;               // weight ring
 constexpr int C3_OFF_W = C3_IO_BUFS * C3_RAW;
 constexpr int C3_OFF_BAR = C3_OFF_W + C3_WBYTES;
 constexpr int C3_SMEM = C3_OFF_BAR + 512 /*barriers*/;
 
 struct C3Layer {
-  const float* wpack;      // tc_pack_layers layout (16-wide chunks of [hi | lo] images)
+  const float* wpack;      // tc_pack_layers layout, pack format 1 (32-wide stages of [tf32 hi | bf16 (hi ; lo)])
   const float* bias;       // [N] or null
   const float* row_scale;  // [V] or null (last layer only)
   int K, N, relu;
@@ -69,21 +72,19 @@ struct C3Layer {
 struct C3Params {
   C3Layer layer[DN_MAX_LAYERS];
   int n_layers, nsrc;
-  int passes;      // 1: one TF32 MMA per product | 3: 3xTF32 (lo*hi + hi*lo + hi*hi) | 2: TF32 hi*hi + bf16 corrections
-  int fmt;         // packed-weight layout (DnLayer::pack_fmt): passes 3 needs 0, passes 2 needs 1, passes 1 takes either
+  int passes;      // 1: one TF32 MMA per product | 2: TF32 hi*hi + bf16 corrections
   int src_width[DN_MAX_SRC];
   int nbuf;        // accumulator buffers (2: ping-pong, column 128 * (g & 1); 1: column 0)
   int ring_col;    // first TMEM column of the operand ring
   int ns_shift;    // log2(ring depth): 2 -> 4 stages (32 KiB weight slots), 1 -> 2 stages (64 KiB weight slots)
-  int nr_shift;    // log2(row-box slots): 2 or 1;  output staging buffers = nio - slots
   // linear head behind the LAST layer (DnLayer::head_*): its N-wide output row is consumed in registers, not stored
   const float* head_w;
   const float* head_b;
   float* head_out;
   int64_t ld_head_out;
   int head_n;
-  int nio;         // 16 KiB row-box + staging buffers in front of the weight ring: 6 (weight ring 128 KiB) or 8 (96 KiB)
-  int pair;        // 1: the MMA warp takes ring stages in pairs (4-slot rings only)
+  int nio;         // 16 KiB row-box + staging buffers in front of the weight ring: 6 (weight ring 128 KiB) or 8 (96 KiB);
+                   //   output staging buffers = nio - C3_RAW_SLOTS
   int64_t V;
   long long* trace;   // optional (tools/trace_chain3.py): per-warp (event, clock64) pairs of CTA 0
   const int32_t* tile_group;   // optional (mesh batches): layer 0 of tile t streams the packed matrix number tile_group[t]
@@ -159,9 +160,9 @@ rows_chain3_kernel(const __grid_constant__ C3Params p, const __grid_constant__ C
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t smem0 = smem_u32(smem);
   if (smem0 & 1023u) __trap();                                          // SWIZZLE_128B boxes need 1024 B alignment
-  const uint32_t nr_sh = (uint32_t)p.nr_shift, nr_mask = (1u << nr_sh) - 1u;
-  const uint32_t nout = (uint32_t)p.nio - (1u << nr_sh), nout_mask = nout - 1u;        // 2 or 4
-  const uint32_t raw_u = smem0, out_u = smem0 + ((uint32_t)C3_RAW << nr_sh), w_u = smem0 + (uint32_t)p.nio * C3_RAW;
+  const uint32_t nr_sh = C3_RAW_SHIFT, nr_mask = C3_RAW_SLOTS - 1;
+  const uint32_t nout = (uint32_t)p.nio - C3_RAW_SLOTS, nout_mask = nout - 1u;        // 2 or 4
+  const uint32_t raw_u = smem0, out_u = smem0 + (uint32_t)C3_RAW * C3_RAW_SLOTS, w_u = smem0 + (uint32_t)p.nio * C3_RAW;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C3_OFF_BAR);
 
   // bars: raw_full[4] raw_empty[4] full[4] ab_empty[4] dm_full[2] do_full[2] dm_empty[2] do_empty[2] res[4 warps][2] done
@@ -264,7 +265,7 @@ rows_chain3_kernel(const __grid_constant__ C3Params p, const __grid_constant__ C
         const uint32_t d_tmem = tmem_base + buf * 128u;
         const uint32_t b_lbo = (uint32_t)N * 16u;
         const uint64_t tmplB = make_desc(0, b_lbo, 128);
-        const uint32_t b_img_u = ((uint32_t)N * 64u) >> 4, b_ks_u = (2u * b_lbo) >> 4, b_chunk_u = 2u * b_img_u;
+        const uint32_t kg2 = (2u * b_lbo) >> 4;           // k-group stride of both stage images (N * 16 B)
         // the previous user of this accumulator must have been drained by everyone who reads it
         C3_TRACE(23);
         if (pend & (1u << buf)) {
@@ -282,7 +283,7 @@ rows_chain3_kernel(const __grid_constant__ C3Params p, const __grid_constant__ C
         // is shallow, `tcgen05.mma` issue blocks for about the execution time) is then paid once per 16 MMAs instead of
         // once per 8, while the operand warps fill the other two slots.  (A 128x128x8 MMA retires in 64 cycles when MMAs
         // are issued back to back, tools/ubench/ubench3.cu: 8 per stage = 512 cycles against ~1100 measured per stage.)
-        const int step = (p.pair && ns_sh == 2) ? 2 : 1;
+        const int step = (ns_sh == 2) ? 2 : 1;
         for (int c = 0; c < nst; c += step, i += (uint32_t)step) {
           C3_TRACE(20);
           for (int h = 0; h < step; ++h) mbar_wait(full + 8 * ((i + (uint32_t)h) & ns_mask), ((i + (uint32_t)h) >> ns_sh) & 1u);
@@ -294,33 +295,17 @@ rows_chain3_kernel(const __grid_constant__ C3Params p, const __grid_constant__ C
               const int cc = c + h;
               const uint32_t a0 = tmem_base + (uint32_t)p.ring_col + s * 64u;
               const uint64_t dbs = tmplB + (w_u4 + s * (w_slot >> 4));
-              if (p.passes == 2) {
-                // stage = [tf32 hi image | bf16 (hi ; lo) image], k-group stride N * 16 B in both.  Four TF32 MMAs (K = 8)
-                // form hi*hi; four bf16 MMAs (K = 16) add the corrections [x_lo | x_hi] . [W_hi ; W_lo] -- 8 instructions
-                // and 32 KiB of shared-memory operand reads per stage where 3xTF32 needs 12 and 48 KiB, same fp32-grade result
-                const uint32_t kg2 = (2u * b_lbo) >> 4;
+              // stage = [tf32 hi image | bf16 (hi ; lo) image].  Four TF32 MMAs (K = 8) form hi*hi; with two passes four
+              // bf16 MMAs (K = 16) add the corrections [x_lo | x_hi] . [W_hi ; W_lo] -- 8 instructions and 32 KiB of
+              // shared-memory operand reads per stage where 3xTF32 needs 12 and 48 KiB, same fp32-grade result
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks)
-                  mma_tf32_ts(d_tmem, a0 + ks * 8, dbs + (uint32_t)ks * kg2, idesc, (cc | ks) ? 1u : 0u);
+              for (int ks = 0; ks < 4; ++ks)
+                mma_tf32_ts(d_tmem, a0 + ks * 8, dbs + (uint32_t)ks * kg2, idesc, (cc | ks) ? 1u : 0u);
+              if (p.passes == 2) {
                 const uint64_t db16 = dbs + (((uint32_t)N * 128u) >> 4);
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
                   mma_f16_ts(d_tmem, a0 + 32 + j * 8, db16 + (uint32_t)j * kg2, idesc16, 1u);
-              } else {
-#pragma unroll
-                for (int ks = 0; ks < C3_KS / 8; ++ks) {
-                  const uint32_t a_hi = a0 + ks * 8, a_lo = a_hi + 32;
-                  const uint64_t b_h = p.fmt ? dbs + (uint32_t)ks * b_ks_u
-                                             : dbs + (uint32_t)(ks >> 1) * b_chunk_u + (uint32_t)(ks & 1) * b_ks_u;
-                  const uint32_t acc = (cc | ks) ? 1u : 0u;
-                  if (p.passes == 3) {
-                    mma_tf32_ts(d_tmem, a_lo, b_h, idesc, acc);
-                    mma_tf32_ts(d_tmem, a_hi, b_h + b_img_u, idesc, 1u);
-                    mma_tf32_ts(d_tmem, a_hi, b_h, idesc, 1u);
-                  } else {
-                    mma_tf32_ts(d_tmem, a_hi, b_h, idesc, acc);
-                  }
-                }
               }
               mma_commit(ab_empty + 8 * s);           // frees TMEM operand stage s and weight stage s
             }
@@ -379,7 +364,6 @@ rows_chain3_kernel(const __grid_constant__ C3Params p, const __grid_constant__ C
 #pragma unroll
           for (int j = 0; j < 16; ++j) split_tf32_fast(x[16 * h + j], hi[j], lo[j]);
           tmem_st16(ta + 16 * h, hi);
-          if (p.passes == 3) tmem_st16(ta + 32 + 16 * h, lo);
         }
       }
       tmem_st_wait();
@@ -737,17 +721,8 @@ int g_attr_dev[kMaxDev];     // 0: not tried, 1: ok, -1: failed
 
 }  // namespace
 
-bool tc_chain3_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("DN_TC_CHAIN3");
-    on = (!e || atoi(e) != 0) ? 1 : 0;
-  }
-  return on == 1;
-}
-
 int tc_chain3_supported(const DnRowsSrc& src, const DnLayer* layers, int n_layers) {
-  if (!tc_chain3_enabled() || tma_encode_fn() == nullptr) return DN_ERR_UNSUPPORTED;
+  if (tma_encode_fn() == nullptr) return DN_ERR_UNSUPPORTED;
   if (n_layers < 1 || n_layers > DN_MAX_LAYERS) return DN_ERR_UNSUPPORTED;
   int k0 = 0;
   for (int s = 0; s < src.nsrc; ++s) {
@@ -810,11 +785,9 @@ int tc_rows_chain3(const DnRowsSrc& src, const DnLayer* layers, int n_layers, in
   memset(&p, 0, sizeof(p));
   memset(&maps, 0, sizeof(maps));
   p.n_layers = n_layers;
-  p.passes = passes;
   for (int l = 0; l < n_layers; ++l)
-    if (layers[l].pack_fmt != layers[0].pack_fmt) return DN_ERR_INVALID_ARGUMENT;
-  p.fmt = layers[0].pack_fmt;
-  if (p.fmt == 1) p.passes = (passes == 3) ? 2 : 1;                 // stage layout [tf32 hi | bf16 (hi ; lo)]
+    if (layers[l].pack_fmt != 1) return DN_ERR_INVALID_ARGUMENT;   // stage layout [tf32 hi | bf16 (hi ; lo)]
+  p.passes = (passes == 3) ? 2 : 1;
 
   p.V = V;
   p.trace = trace;
@@ -852,25 +825,10 @@ int tc_rows_chain3(const DnRowsSrc& src, const DnLayer* layers, int n_layers, in
   if (nmax <= 128) { p.nbuf = 2; p.ring_col = 256; p.ns_shift = 2; }
   else if (n_layers == 2) { p.nbuf = 2; p.ring_col = 384; p.ns_shift = 1; }
   else { p.nbuf = 1; p.ring_col = 256; p.ns_shift = 1; }
-  // output-heavy chains (few layer-0 stages per tile, many output columns): 2 row-box slots + 4 staging buffers
-  // (measured on the from_basis -> [P|Q] chain: 2 + 4 was SLOWER, 124 vs 108 us -- the extra staging traffic competes
-  //  with the tensor core for shared-memory bandwidth -- so 4 + 2 stays the default; DN_C3_NR=2 selects 2 + 4)
-  p.nr_shift = 2;
   p.nio = C3_IO_BUFS;
-  {
-    static int pair_env = -1;
-    if (pair_env < 0) { const char* e = getenv("DN_C3_PAIR"); pair_env = e ? atoi(e) : 1; }
-    p.pair = pair_env;
-  }
   if (n_layers == 1 && layers[0].dots_src && nmax <= 128) {
     // complex-dots layer: 4 row boxes + 4 staging buffers (all gX / gY boxes of a tile prefetched) + a 2-stage ring
     p.nio = 8; p.ns_shift = 1;
-  }
-  {
-    static int nr_env = -2;
-    if (nr_env == -2) { const char* e = getenv("DN_C3_NR"); nr_env = e ? atoi(e) : -1; }
-    if (nr_env == 2) p.nr_shift = 1;
-    if (nr_env == 4) p.nr_shift = 2;
   }
 
   const int64_t ntiles = (V + C3_TILE - 1) / C3_TILE;

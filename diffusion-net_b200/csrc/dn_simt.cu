@@ -8,7 +8,6 @@
 #include "dn_internal.h"
 #include "dn_tc_ptx.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace {
 
@@ -963,14 +962,9 @@ int launch_spmm_features(const dn_csr* g, const float* xd, const float* pq, int 
                          float* feat, cudaStream_t st) {
   if (V <= 0) return DN_OK;
   if (C % 4) return DN_ERR_UNSUPPORTED;
-  static int use_patch = -1;
-  if (use_patch < 0) {
-    const char* e = getenv("DN_SPMM_PATCH");
-    use_patch = e ? atoi(e) : 1;
-  }
   // C == 128 only: that is the shape validated on the GPU (bit-identical to the plain kernel, both ROT variants); the
   // phase-2 shuffles also assume every lane owns a float4 of the row (C/4 a multiple of 32)
-  if (g->patches && use_patch && g->patches->n_patches > 0 && C == 128) {
+  if (g->patches && g->patches->n_patches > 0 && C == 128) {
     const dn_patches& P = *g->patches;
     const int ld = rotations ? 2 * C : C;
     const size_t smem = (size_t)P.max_src * (size_t)(C + ld) * 4;
@@ -990,12 +984,9 @@ int launch_spmm_features(const dn_csr* g, const float* xd, const float* pq, int 
     }
   }
   const float2* vals = reinterpret_cast<const float2*>(g->vals);
-  static int use_blk = -1;
-  if (use_blk < 0) {
-    const char* e = getenv("DN_SPMM_BLK");
-    use_blk = e ? atoi(e) : 1;   // measured (tools/ab_gather.py, V=200k): 1 -> 174 us (282 permuted) vs 181 (347) for the warp-per-row kernel
-  }
-  if ((C == 128 || C == 256) && use_blk) {
+  // block gather at C = 128 / 256: measured (profiles/r02_ab_gather_blk.log, V=200k) 175 us (281 permuted) vs 181 (347)
+  // for the warp-per-row kernel below, which serves the other widths
+  if (C == 128 || C == 256) {
     const unsigned ctas = (unsigned)((V + GB_ROWS - 1) / GB_ROWS);
     const int ld = rotations ? 2 * C : C;
 #define DN_BLK_LAUNCH(ROT_, NH_) \

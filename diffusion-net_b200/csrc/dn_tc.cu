@@ -1169,7 +1169,8 @@ static long long* take_trace_ptr() {
   return nullptr;   // already used once
 }
 
-// declared in dn_chain.cu
+// declared in dn_chain.cu.  tc_rows_chain3 takes weights in pack format 1 only (DN_ERR_INVALID_ARGUMENT otherwise):
+// passes 3 runs TF32 hi*hi plus bf16 correction terms, passes 1 the TF32 hi*hi term alone
 int tc_chain3_supported(const DnRowsSrc& src, const DnLayer* layers, int n_layers);
 int tc_rows_chain3(const DnRowsSrc& src, const DnLayer* layers, int n_layers, int64_t V, int passes, int sm_count,
                    long long* trace, cudaStream_t st);
@@ -1218,11 +1219,6 @@ bool tc_supported_device() {
   return d && d->ok == 1;
 }
 
-static bool ts_allowed_env() {
-  const char* e = getenv("DN_TC_TS");
-  return !e || atoi(e) != 0;
-}
-
 // shapes the round-1 kernels (rows_chain_kernel / rows_chain_ts_kernel) take
 static int tc_rows_chain_legacy_supported(const DnRowsSrc& src, const DnLayer* layers, int n_layers) {
   if (n_layers < 1 || n_layers > DN_MAX_LAYERS) return DN_ERR_UNSUPPORTED;
@@ -1243,7 +1239,7 @@ static int tc_rows_chain_legacy_supported(const DnRowsSrc& src, const DnLayer* l
     if (l > 0 && L.K != layers[l - 1].N) return DN_ERR_UNSUPPORTED;
     // a 256-wide accumulator cannot ping-pong with another one; the TMEM-A kernel still fits the two-layer
     // pattern (N0 <= 128 then N1 <= 256: from_basis -> [P|Q]) next to a 4-stage activation ring
-    if (L.N > 128 && n_layers > 1 && !(ts_allowed_env() && n_layers == 2 && l == 1 && layers[0].N <= 128))
+    if (L.N > 128 && n_layers > 1 && !(n_layers == 2 && l == 1 && layers[0].N <= 128))
       return DN_ERR_UNSUPPORTED;
   }
   if (!layers[n_layers - 1].out) return DN_ERR_UNSUPPORTED;
@@ -1256,17 +1252,8 @@ int tc_rows_chain_supported(const DnRowsSrc& src, const DnLayer* layers, int n_l
   return tc_rows_chain_legacy_supported(src, layers, n_layers);
 }
 
-static bool hybrid_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("DN_TC_HYBRID");
-    on = (!e || atoi(e) != 0) ? 1 : 0;
-  }
-  return on == 1;
-}
-
 void tc_choose_pack_fmt(const DnRowsSrc& src, DnLayer* layers, int n_layers, int passes) {
-  int fmt = (hybrid_enabled() && tc_chain3_supported(src, layers, n_layers) == DN_OK) ? 1 : 0;
+  int fmt = tc_chain3_supported(src, layers, n_layers) == DN_OK ? 1 : 0;
   if (passes == DN_PASSES_BF16 && tc_chain16_supported(src, layers, n_layers) == DN_OK) fmt = 2;
   for (int l = 0; l < n_layers; ++l) layers[l].pack_fmt = fmt;
 }
@@ -1402,16 +1389,9 @@ int tc_rows_chain(const DnRowsSrc& src, const DnLayer* layers_in, int n_layers, 
   p.acc_col[0] = 0; p.acc_col[1] = 128; p.nbuf = 2; p.a_col0 = 256; p.nsa = 8;
   if (p.nmax == 256 && n_layers == 1) { p.acc_col[1] = 0; p.nbuf = 1; }
   if (p.nmax == 256 && n_layers == 2) { p.a_col0 = 384; p.nsa = 4; }   // [0,128) | [128,384) | ring [384,512)
-  {
-    // measured (V=200k): role specialisation wins on the 2-layer from_basis+[P|Q] chain (196 -> 167 us: few
-    // layer-0 chunks, heavy epilogues) and loses on the MiniMLP (270 -> 280 us: 24 layer-0 chunks per tile)
-    static int split_env = -2;
-    if (split_env == -2) {
-      const char* e = getenv("DN_TC_SPLIT");
-      split_env = e ? atoi(e) : -1;
-    }
-    p.ts_split = split_env >= 0 ? split_env : (n_layers == 2 ? 1 : 0);
-  }
+  // measured (V=200k): role specialisation wins on the 2-layer from_basis+[P|Q] chain (196 -> 167 us: few
+  // layer-0 chunks, heavy epilogues) and loses on the MiniMLP (270 -> 280 us: 24 layer-0 chunks per tile)
+  p.ts_split = (n_layers == 2) ? 1 : 0;
   for (int l = 0; l < n_layers; ++l) {
     const DnLayer& L = layers[l];
     TcLayer& T = p.layer[l];
@@ -1419,12 +1399,7 @@ int tc_rows_chain(const DnRowsSrc& src, const DnLayer* layers_in, int n_layers, 
     T.out = L.out; T.ld_out = L.ld_out; T.K = L.K; T.N = L.N; T.relu = L.relu;
   }
   const int64_t ntiles = (V + TILE_M - 1) / TILE_M;
-  static int use_ts = -1;
-  if (use_ts < 0) {
-    const char* e = getenv("DN_TC_TS");
-    use_ts = e ? atoi(e) : 2;   // 0: never, 1: always, 2 (default): for chained layers
-  }
-  if (use_ts == 1 || (use_ts == 2 && n_layers > 1)) {   // activations in TMEM (A operand read from tensor memory), one CTA per SM
+  if (n_layers > 1) {   // chained layers: activations in TMEM (A operand read from tensor memory), one CTA per SM
     const int grid1 = (int)(ntiles < dv->sms ? ntiles : dv->sms);
     rows_chain_ts_kernel<<<grid1, TS_THREADS, TS_SMEM, st>>>(p);
     DN_LAUNCH_CHECK();

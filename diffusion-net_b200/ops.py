@@ -181,7 +181,7 @@ class GradOperators:
         rows = torch.repeat_interleave(torch.arange(self.V, device=self.device), counts)
         return float(((colidx[:self.nnz].long() - rows).abs() <= 8).float().mean())
 
-    def build_patches(self, max_targets=None, max_src=None):
+    def build_patches(self, max_targets=32, max_src=72):
         """Locality structure for the fused gradient-features kernel (``dn_patches``): rows are clustered into patches of
         graph-adjacent vertices (host side, ``dn_patch_build``) so the kernel stages each patch's distinct neighbour
         rows in shared memory once.  Worth its one-off cost (a D2H of the pattern, the clustering, an H2D) only for
@@ -191,8 +191,6 @@ class GradOperators:
         if getattr(self, "_patches", None) is not None or self.nnz == 0:
             return self
         import numpy as np
-        max_targets = int(os.environ.get("DN_PATCH_T", 32)) if max_targets is None else max_targets
-        max_src = int(os.environ.get("DN_PATCH_R", 72)) if max_src is None else max_src
         st, rowptr, colidx, vals = self.csr
         rp = rowptr.cpu().numpy()
         ci = colidx[:self.nnz].cpu().numpy()
@@ -257,20 +255,19 @@ class GradOperators:
 
 
 _prep_cache = {}
-# dn_patches policy on the SECOND use of an operator pair (= the operators are resident): "auto" (default) builds the
-# structure only for poorly ordered meshes, "1" always, "0" never.  Measured on B200 (tools/ab_patch.py, V = 200k,
-# C = 128): the staged gather takes ~206 us whatever the vertex order; the plain gather takes 179 us on a mesh whose
-# order has locality (47 % L1 hits) and 346 us on a randomly permuted one.
-auto_patch = os.environ.get("DN_SPMM_PATCH", "auto")
+# dn_patches policy on the SECOND use of an operator pair (= the operators are resident): the structure is built only
+# for poorly ordered meshes.  Measured on B200 (tools/ab_patch.py, V = 200k, C = 128): the staged gather takes ~206 us
+# whatever the vertex order; the plain gather takes 179 us on a mesh whose order has locality (47 % L1 hits) and
+# 346 us on a randomly permuted one.
 PATCH_LOCALITY_THRESHOLD = 0.25
 
 
 def _maybe_patch(ops):
-    if auto_patch == "0" or getattr(ops, "_patches", None) is not None:
+    if getattr(ops, "_patches", None) is not None:
         return
     if torch.cuda.is_current_stream_capturing():     # the decision needs host round trips: not inside a graph capture
         return
-    if auto_patch == "1" or ops.locality() < PATCH_LOCALITY_THRESHOLD:
+    if ops.locality() < PATCH_LOCALITY_THRESHOLD:
         ops.build_patches()
     else:
         ops._patches = False            # decided: the vertex order already has locality

@@ -5,6 +5,7 @@ Tolerance: north_star asks for 1e-5 relative fp32; the metric is max|ours - gold
 (SURVEY.md section 8c).  TOL below is that bound; the exact-fp32 SIMT engine is held to 2e-6.
 """
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -261,6 +262,86 @@ def test_errors_and_no_cpu_fallback(dn):
         dn.DiffusionNet(3, 4, outputs_at="nowhere")
     with pytest.raises(ValueError, match="C_in=3"):
         dn.DiffusionNet(3, 4, C_width=32).cuda()(torch.zeros(10, 4).cuda(), torch.ones(10).cuda())
+
+
+_NOT_SM100_SCRIPT = r'''
+import ctypes as C, sys, types
+sys.path.insert(0, %r)
+import torch
+import diffusion_net_b200 as dn
+from diffusion_net_b200 import _lib, ops
+lib = _lib.load()
+assert dn.get_engine() == "tc3x"
+K = W = 64
+mass, L, evals, evecs, gX, gY = dn.synthetic.structural_operators(12, 16, K, seed=0, device="cuda")
+V = mass.shape[0]
+g = torch.Generator().manual_seed(0)
+rnd = lambda *s: torch.randn(*s, generator=g).cuda()
+x, spec, time = rnd(V, W), rnd(K, W), torch.full((W,), 0.1, device="cuda")
+A_re, A_im, pq, hidden = rnd(W, W), rnd(W, W), rnd(V, 2 * W), [rnd(V, W), rnd(V, W)]
+wts, bias = [rnd(W, 3 * W), rnd(W, W), rnd(W, W)], [rnd(W), rnd(W), rnd(W)]
+head = (rnd(4, W), rnd(4))
+gops = ops.GradOperators(gX, gY)
+gops.csr_t
+mb = dn.MeshBatch([dict(mass=mass, evals=evals, evecs=evecs, gradX=gops)] * 2)
+xb, specb = rnd(mb.V, W), rnd(2, K, W)
+out, gA_re, gA_im = torch.empty_like(x), rnd(W, W), rnd(W, W)
+outb = torch.empty_like(xb)
+ws = ops.workspace(mb.V, K, 3 * W, x.device, extra=2 * K * W * 12)
+prm = _lib.dn_block_params(time.data_ptr(), A_re.data_ptr(), A_im.data_ptr(), 1, 1, 3,
+                           _lib.ptr_array([w.data_ptr() for w in wts]), _lib.ptr_array([b.data_ptr() for b in bias]),
+                           _lib.int_array([3 * W, W, W, W]))
+ctx = types.SimpleNamespace
+calls = {
+    "dn_to_basis": lambda: ops.to_basis_raw(x, evecs, mass),
+    "dn_from_basis": lambda: ops.from_basis_raw(spec, evecs),
+    "dn_learned_time_diffusion_fwd": lambda: ops.DiffusionFn.apply(x, time, mass, evals, evecs),
+    "dn_learned_time_diffusion_bwd": lambda: ops.DiffusionFn.backward(ctx(saved_tensors=(mass, evals, evecs, time, spec)), x),
+    "dn_learned_time_diffusion_fwd_batched": lambda: ops.BatchedDiffusionFn.apply(xb, time, mb),
+    "dn_learned_time_diffusion_bwd_batched": lambda: ops.BatchedDiffusionFn.backward(
+        ctx(batch=mb, saved_tensors=(time, specb)), xb),
+    "dn_gradient_features_fwd": lambda: ops.GradFeaturesFn.apply(x, A_re, A_im, gops),
+    "dn_gradient_features_bwd": lambda: _lib.check(lib.dn_gradient_features_bwd(
+        C.byref(gops.csr[0]), C.byref(gops.csr_t[0]), x.data_ptr(), x.data_ptr(), pq.data_ptr(), x.data_ptr(),
+        A_re.data_ptr(), A_im.data_ptr(), 1, V, W, out.data_ptr(), gA_re.data_ptr(), gA_im.data_ptr(), ws.data_ptr(),
+        ws.numel(), ops._engine, ops._stream()), "dn_gradient_features_bwd"),
+    "dn_mini_mlp_fwd": lambda: ops.mlp_apply([x, x, x], wts, bias, residual=x),
+    "dn_mini_mlp_bwd": lambda: ops.MLPFn.backward(ctx(meta=(3, 3, True, [3 * W, W, W, W], [True] * 3),
+                                                      saved_tensors=(x, x, x, *wts, *hidden), n_hidden=2, n_masks=0), x),
+    "dn_block_fwd": lambda: ops.block_forward_raw(x, mass, evals, evecs, gops, time, A_re, A_im, wts, bias, True),
+    "dn_block_fwd_profile": lambda: ops.block_forward_raw(x, mass, evals, evecs, gops, time, A_re, A_im, wts, bias, True,
+                                                          profile=[]),
+    "dn_block_fwd_ex (head)": lambda: ops.block_forward_raw(x, mass, evals, evecs, gops, time, A_re, A_im, wts, bias,
+                                                            True, head=head),
+    "dn_block_fwd_ex (batch)": lambda: dn.batch.block_forward_batched_raw(mb, xb, time, A_re, A_im, wts, bias, True),
+    "dn_block_fwd_batched": lambda: _lib.check(lib.dn_block_fwd_batched(
+        xb.data_ptr(), mb.mass.data_ptr(), mb.evals.data_ptr(), mb.evecs.data_ptr(), C.byref(mb.gops.csr[0]),
+        C.byref(prm), C.byref(mb.desc), mb.V, K, W, outb.data_ptr(), ws.data_ptr(), ws.numel(), ops._engine,
+        ops._stream()), "dn_block_fwd_batched"),
+}
+torch.cuda.synchronize()
+bad = []
+for name, fn in calls.items():
+    n0 = lib.dn_kernel_launch_count()
+    try:
+        fn()
+        err = "returned normally"
+    except RuntimeError as e:
+        err = repr(e)
+    launched = lib.dn_kernel_launch_count() - n0
+    if "(-4)" not in err or launched:
+        bad.append("{}: {}, {} kernels enqueued".format(name, err, launched))
+print("\n".join(bad) if bad else "ALL_NOT_SM100")
+'''
+
+
+def test_tensor_core_engine_on_unsupported_device_enqueues_nothing(dn):
+    """With tcgen05 unavailable (DN_TC_DISABLE=1), every tensor-core-capable entry point under the tc3x engine fails
+    with DN_ERR_NOT_SM100 before it enqueues a kernel: no silent SIMT fallback and no partial work on the stream."""
+    env = dict(os.environ, DN_TC_DISABLE="1", DN_B200_ENGINE="tc3x")
+    r = subprocess.run([sys.executable, "-c", _NOT_SM100_SCRIPT % ROOT], capture_output=True, text=True, timeout=600,
+                       env=env)
+    assert r.returncode == 0 and r.stdout.strip().endswith("ALL_NOT_SM100"), r.stdout + r.stderr
 
 
 def _structural_case(dn, n, m, K, C, seed=0, **kw):
@@ -808,8 +889,9 @@ def test_full_size_hks_and_transpose_properties(dn):
 
 @pytest.mark.parametrize("permute", [False, True])
 @pytest.mark.parametrize("rot", [True, False])
-def test_patched_gather_is_bit_identical(dn, permute, rot):
-    """dn_patches (shared-memory staged gather) vs the plain gather kernel: same entries, same order, same arithmetic."""
+def test_patched_gather_is_bit_identical_and_patch_policy(dn, permute, rot):
+    """dn_patches (shared-memory staged gather) vs the plain gather kernel: same entries, same order, same arithmetic;
+    and prepare_operators builds the structure on the second use exactly when the vertex order lacks locality."""
     dn.set_engine("tc3x")
     C = 128
     mass, L, evals, evecs, gX, gY = dn.synthetic.structural_operators(60, 70, 32, seed=2, device="cuda", permute=permute)
@@ -831,8 +913,7 @@ def test_patched_gather_is_bit_identical(dn, permute, rot):
     assert getattr(o1, "_patches", None) is None
     o2 = dn.ops.prepare_operators(gX, gY)
     assert o2 is o1
-    if dn.ops.auto_patch == "auto":
-        # (a symmetric permutation keeps the diagonal entry on the diagonal: 1/7 of the entries stay 'local')
-        assert (o2.locality() < 0.2 and o2._patches) if permute else (o2.locality() > 0.3 and o2._patches is False)
-        with torch.no_grad():
-            assert torch.equal(dn.ops.GradFeaturesFn.apply(xd, A_re, A_im, o2), ref)
+    # (a symmetric permutation keeps the diagonal entry on the diagonal: 1/7 of the entries stay 'local')
+    assert (o2.locality() < 0.2 and o2._patches) if permute else (o2.locality() > 0.3 and o2._patches is False)
+    with torch.no_grad():
+        assert torch.equal(dn.ops.GradFeaturesFn.apply(xd, A_re, A_im, o2), ref)

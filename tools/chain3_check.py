@@ -2,8 +2,7 @@
 for the two fused chains of the block (from_basis + [P|Q]; MiniMLP + skip) and single layers, at several V
 (ragged last tile, V < 128, one tile, many tiles per CTA), repeated calls to catch hand-off races.
 
-    python tools/chain3_check.py            # default path (DN_TC_CHAIN3=1)
-    DN_TC_CHAIN3=0 python tools/chain3_check.py   # the round-1 kernels, for the A/B
+    python tools/chain3_check.py
 """
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -121,7 +120,6 @@ def check_shapes(V=5000):
 
 
 if __name__ == "__main__":
-    print("DN_TC_CHAIN3 =", os.environ.get("DN_TC_CHAIN3", "1 (default)"), flush=True)
     check_shapes()
     for V in (100, 128, 129, 1000, 18944, 18945, 40000):
         print("V={:6d}: {}".format(V, check(V)), flush=True)

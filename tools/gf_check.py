@@ -1,4 +1,4 @@
-"""Tensor-core gradient-features route (DN_GF_TC): per-stage times of the fused block at V=200k, the x-only gather's
+"""Tensor-core gradient-features route (C_width = 128 with rotations): per-stage times of the fused block at V=200k, the x-only gather's
 share of stage [4], parity vs the exact engine, repeatability."""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

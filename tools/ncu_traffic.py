@@ -10,8 +10,8 @@ raw = subprocess.run(["ncu", "-i", rep, "--page", "raw", "--csv"], capture_outpu
 rows = list(csv.reader(raw.splitlines()))
 hdr, units = rows[0], rows[1]
 ix = {h: i for i, h in enumerate(hdr)}
-# launch sequence of dn_block_fwd at C = 128 with the tensor-core gradient features (DN_GF_TC=1, default); with
-# DN_GF_TC=0 pass "commuted" as third argument
+# launch sequence of dn_block_fwd at C = 128 with the tensor-core gradient features; for a capture of the commuted
+# route (C_width != 128, no rotations, the bf16 engine, patched operators) pass "commuted" as third argument
 STAGE = [("to_basis_kernel", "to_basis"), ("pack_weights_kernel", "pack_weights"), ("rows_chain", "from_basis_pq"),
          ("spmm_gxy", "grad_gather_x"), ("rows_chain", "grad_dots_gemm"), ("rows_chain", "grad_dots_gemm_2"), ("rows_chain", "mlp")]
 if len(sys.argv) > 3 and sys.argv[3] == "commuted":
